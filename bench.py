@@ -20,6 +20,15 @@
 --impl reference times the CPU restatement of the reference env (oracle/, kind "port": the reference's own native
 modules are not shipped, DESIGN.md) on all host cores over a bounded sample of the same workload.  That arm never loads
 the product package or its library.
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step returned to its caller as DIR/<name>.npy
+(float32, or float64 where an integer needs it): for a fixed seeded sample of the envs (config 5: pairs) the step
+results r / done / cat / reward, the face and the legal moves of the new state (one-hot rows and count per env; config 3
+also the Q-values of the scored lists with their counts, and the chosen move index of the step; config 5 the move lists
+as per-rank card counts).  Lists are written whole: the sample ends before the first env whose lists would pass the row
+limit, and env_index (pair_index) lists the envs written.  The inputs are seeded, so two builds run with the same
+arguments can be compared output for output.  Under torchrun every rank writes its own share of the sample with a
+_rank<r> suffix; all ranks together stay within 64 MB.
 """
 import argparse
 import importlib.util
@@ -78,7 +87,13 @@ def parse_args():
                     help="config 3: how the landlord's legal moves are scored -- fused: ddz_q_features (the network's first layer "
                          "from the packed state and lists, no input tensor) + two library GEMMs; module: the torch module on the "
                          "[n, C+1, 15, 4] input written by ddz_encode_state_actions")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (a fixed sample, at most 64 MB) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     if args.envs is None:
         args.envs = {2: 4096, 3: 65536}.get(args.config, 131072)
     if args.groups is None:
@@ -330,6 +345,68 @@ def all_ranks_ok(D, torch, dev, world, verdict):
     return verdict if verdict != "ok" else ("ok" if int(bad.item()) == 0 else "MISMATCH on another rank")
 
 
+# ---------------------------------------------------------------------------------------------- --dump-outputs
+# The limits are for all ranks together: under torchrun each rank dumps 1/world of the sample and of the rows.
+DUMP_BYTES = 64 << 20               # all arrays of one dump, over all ranks
+DUMP_ENVS = 8192                    # sampled envs: 17.7 MB of face
+DUMP_ROWS = 1 << 16                 # legal-move rows of the sampled envs (15.7 MB of one-hots; 5-8 moves per env in configs 3/4)
+DUMP_PAIRS = 1024                   # config 5: sampled pairs (~140 moves each)
+DUMP_MOVES = 1 << 18                # ... and their moves as 15 card counts each (15.7 MB)
+
+
+def dump_sample(n, k, limit, *offsets):
+    """sorted indices of the envs (pairs) of n whose outputs are dumped: k of them drawn with a fixed seed (the same in
+    every run of the same size), then only the leading ones whose lists, under every CSR offsets given (host int [n+1]),
+    hold at most `limit` rows together -- lists are dumped whole, never cut"""
+    import numpy as np
+    idx = np.arange(n) if n <= k else np.sort(np.random.default_rng(SEED).choice(n, k, replace=False))
+    keep = len(idx)
+    for off in offsets:
+        keep = min(keep, int(np.searchsorted(np.cumsum(off[idx + 1] - off[idx]), limit, side="right")))
+    return idx[:keep]
+
+
+def list_rows(offsets, idx):
+    """indices of the rows of the CSR lists idx (offsets: host int [n+1]), in list order"""
+    import numpy as np
+    return np.concatenate([np.arange(offsets[i], offsets[i + 1], dtype=np.int64) for i in idx] + [np.zeros(0, np.int64)])
+
+
+def batch_offsets(torch, envs):
+    """host int64 [B+1]: the legal-move offsets of the batch the env objects `envs` (the groups of a GroupedEnv, or one
+    env) make together"""
+    import numpy as np
+    counts = torch.cat([e.offsets[1:] - e.offsets[:-1] for e in envs]).cpu().numpy()
+    return np.concatenate([[0], np.cumsum(counts, dtype=np.int64)])
+
+
+def env_outputs(torch, envs, idx, off):
+    """What a caller of the fused env-step holds after it, for the envs idx of the batch `envs` (legal-move offsets off,
+    batch_offsets): the step's r / done / cat / reward, and the new state's face and legal moves (the one-hot rows of the
+    listed envs, in order, and each env's count)."""
+    import numpy as np
+    dev = envs[0].device
+    sel = torch.as_tensor(idx, device=dev)
+    rows = torch.as_tensor(list_rows(off, idx), device=dev)
+    batch = lambda f: torch.cat([f(e) for e in envs])
+    host = lambda t: t.cpu().numpy().astype(np.float32)
+    return {"env_index": idx.astype(np.float64), "r": host(batch(lambda e: e.r)[sel]), "done": host(batch(lambda e: e.done)[sel]),
+            "cat": host(batch(lambda e: e.cat)[sel]), "reward": host(batch(lambda e: e.reward)[sel]),
+            "face": host(batch(lambda e: e.face)[sel]), "legal_counts": np.diff(off)[idx].astype(np.float32),
+            "legal_actions": host(batch(lambda e: e.valid_actions()[0])[rows])}
+
+
+def write_dump(out_dir, arrays, rank, world):
+    import numpy as np
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES // world:
+        raise SystemExit("--dump-outputs: %d bytes on rank %d exceed its share of the %d-byte limit" % (total, rank, DUMP_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ("_rank%d" % rank if world > 1 else "") + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------- config 4
 def run_config4(args):
     import numpy as np
@@ -353,7 +430,8 @@ def run_config4(args):
         ge.rollout_step()
     SPG = args.steps_per_graph if (args.steps_per_graph % 2 == 0 and K % args.steps_per_graph == 0) else 2
     ge.capture(steps_per_graph=SPG)     # the loop is launch-bound from Python: replay SPG steps per group as one CUDA graph
-    for _ in range(max(-(-max(W, 3) // SPG), 2)):
+    warm_replays = max(-(-max(W, 3) // SPG), 2)
+    for _ in range(warm_replays):
         ge.replay()
     ge.join()
     torch.cuda.synchronize(dev)
@@ -413,6 +491,10 @@ def run_config4(args):
     timed_state = None if args.no_verify else (
         torch.cat([e._fields()[0] for e in ge.envs], dim=1).clone(), torch.cat([e._fields()[1] for e in ge.envs]).clone(),
         ge.stats.clone(), int(ge.envs[0]._stepno), sum(int(e.num_actions) for e in ge.envs))
+    if args.dump_outputs:               # before the regions below step the same envs further
+        off = batch_offsets(torch, ge.envs)
+        idx = dump_sample(B, DUMP_ENVS // world, DUMP_ROWS // world, off)
+        write_dump(args.dump_outputs, env_outputs(torch, ge.envs, idx, off), rank, world)
 
     # ---------------- for information: one chain of launches over all envs (no groups), graph replay and eager Python loop
     info = {}
@@ -537,7 +619,8 @@ def run_config4(args):
             "dtype": "u64", "data": "synthetic",
             "config": dict({"workload": workload_text(args), "baseline_config": args.config,
                             "envs_per_gpu": B, "env_groups_per_gpu": NG, "face_channels": CHANNELS, "mean_legal_moves": nbar,
-                            "prefill_steps": args.prefill, "pool_games": P, "parallelism": "env-shard x%d" % world,
+                            "prefill_steps": args.prefill, "warmup_env_steps": warm_replays * SPG, "pool_games": P,
+                            "parallelism": "env-shard x%d" % world,
                             "launch": "CUDA graph replay, %d env-steps per graph, one chain per env group" % SPG,
                             "collectives": ("none (single GPU)" if world == 1 else
                                             "stats all-reduce (int64[16], NCCL LL) %d time(s) in the timed region, every %d steps "
@@ -618,6 +701,13 @@ def run_config5(args):
     e1.record()
     barrier()
     total_ms = e0.elapsed_time(e1)
+    if args.dump_outputs:               # the lists of the last call: per-pair counts, and the moves as per-rank card counts
+        off = gen.offsets.cpu().numpy().astype(np.int64)
+        idx = dump_sample(n, DUMP_PAIRS // world, DUMP_MOVES // world, off)
+        rows = torch.as_tensor(list_rows(off, idx), device=dev)
+        write_dump(args.dump_outputs, {"pair_index": idx.astype(np.float64), "moves_total": np.array([off[n]], np.float64),
+                                       "move_counts": np.diff(off)[idx].astype(np.float32),
+                                       "moves": D.unpack_counts(gen.actions[rows]).cpu().numpy().astype(np.float32)}, rank, world)
 
     # ---------------- e2e: pinned host (hand, last) arrays in, the packed CSR lists (offsets + moves) back in pinned memory
     hh, lh = torch.as_tensor(hands_np.view(np.int64)).pin_memory(), torch.as_tensor(lasts_np.view(np.int64)).pin_memory()
@@ -742,6 +832,7 @@ def run_config3(args):
         env.rollout_step(perm=pd, lord_pile=ld, pool_games=P)
     gen = torch.Generator(device=dev); gen.manual_seed(1)
     scored = [0]
+    last = {}                                              # the last timed step's scores and decisions, for --dump-outputs
 
     def step(timed):
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)] if timed else None
@@ -760,6 +851,8 @@ def run_config3(args):
         if timed:
             ev[2].record()
             scored[0] += int(q.numel())
+            if args.dump_outputs:
+                last.update(q=q, offsets=off, choice=choice)
         return ev
 
     for _ in range(W):
@@ -775,6 +868,16 @@ def run_config3(args):
     total_ms = e0.elapsed_time(e1)
     net_ms = sum(a.elapsed_time(b) for a, b, _ in evs) / K
     env_ms = sum(b.elapsed_time(c) for _, b, c in evs) / K
+    if args.dump_outputs:
+        # + what the step decided on: the Q-values of the sampled envs' moves in the scored (pre-step) lists, 0 where the
+        # landlord is not to move, with each env's count in those lists (q_counts), and the chosen move indices
+        off, off0 = batch_offsets(torch, [env]), last["offsets"].cpu().numpy().astype(np.int64)
+        idx = dump_sample(B, DUMP_ENVS, DUMP_ROWS, off, off0)
+        out = env_outputs(torch, [env], idx, off)
+        out["q_counts"] = np.diff(off0)[idx].astype(np.float32)
+        out["q_values"] = last["q"][torch.as_tensor(list_rows(off0, idx), device=dev)].cpu().numpy().astype(np.float32)
+        out["choice"] = last["choice"][torch.as_tensor(idx, device=dev)].cpu().numpy().astype(np.float32)
+        write_dump(args.dump_outputs, out, 0, 1)
     st = (env.stats - st0).cpu().numpy()
     if int(env.stats[7].item()):
         raise SystemExit("env reported errors")

@@ -1690,3 +1690,48 @@ def test_graph_replay_after_steps_that_bypass_the_device_counter(D, oracle):
     _compare_state(env, ref, t)
     _compare_observation(env, ref, t)
     assert int(env.stats[7].item()) == 0
+
+
+def test_bench_dump_outputs_are_reproducible(D, oracle, tmp_path):
+    """bench.py --dump-outputs: two runs with the same arguments write the same arrays (float32 / float64, a fixed sample
+    of the envs), and they are what the last timed step returned: the oracle, replaying the bench's deals and Philox
+    streams for prefill + warm-up + timed steps, gives the same r / done / cat / reward of that step and the same face
+    and legal lists of the state after it, env by env."""
+    import json
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    import bench
+    B, steps = 12288, 3                                  # more envs than the dump samples
+    dumps = []
+    for run in range(2):
+        out_dir = str(tmp_path / ("run%d" % run))
+        cmd = [sys.executable, os.path.join(root, "bench.py"), "--envs", str(B), "--steps", str(steps), "--warmup", "2",
+               "--prefill", "20", "--no-cpu-baseline", "--no-single", "--clock-interval-ms", "0", "--dump-outputs", out_dir]
+        res = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
+        assert res.returncode == 0, res.stderr[-2000:]
+        line = json.loads(res.stdout.strip().splitlines()[-1])
+        assert line["steps"] == steps and line["verify"] == "ok"
+        dumps.append({f[:-4]: np.load(os.path.join(out_dir, f)) for f in sorted(os.listdir(out_dir))})
+    a, b = dumps
+    assert sorted(a) == ["cat", "done", "env_index", "face", "legal_actions", "legal_counts", "r", "reward"]
+    assert sum(x.nbytes for x in a.values()) <= 64 << 20
+    for name in a:
+        assert a[name].dtype in (np.float32, np.float64) and np.array_equal(a[name], b[name]), name
+    idx = a["env_index"].astype(np.int64)
+    assert len(idx) == bench.DUMP_ENVS and (np.diff(idx) > 0).all() and idx[-1] < B
+    assert a["legal_actions"].shape == (int(a["legal_counts"].sum()), 15, 4)
+
+    P, seed = bench.POOL_GAMES, bench.SEED
+    perm, lord = D.random_deals(B, seed=seed, pool_games=P)
+    ref = oracle.RefBatch(B, variant=bench.VARIANT)
+    ref.deal(perm, lord, pool_games=P)
+    for t in range(line["config"]["prefill_steps"] + line["config"]["warmup_env_steps"] + steps):
+        ref.observe(want_f32=False, want_face=False)
+        r, done, cat, rew = ref.step(mode=2, seed=seed, env0=0, step=t)
+        ref.deal(perm, lord, only_done=True, pool_games=P)
+    off, _, af, face = ref.observe()
+    for name, want in (("r", r), ("done", done), ("cat", cat), ("reward", rew), ("face", face), ("legal_counts", np.diff(off))):
+        assert np.array_equal(a[name], want[idx].astype(np.float32)), name
+    assert np.array_equal(a["legal_actions"], np.concatenate([af[off[i]:off[i + 1]] for i in idx]))
