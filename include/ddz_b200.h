@@ -174,8 +174,8 @@ int ddz_playout(void* state, int max_steps, uint64_t seed, uint64_t env0, uint32
  * [n, C+1, 15, 4] input of net.py:87-90.
  * Every input plane is a function of one nibble per rank, so the convolutions are sums of table rows:
  * rank_tables float32 [C+1][16][W][4] (T[c][nibble][o][k] = sum_{j<=k} W_k+1[o,c,0,j] * slot_j(nibble); the row of nibble 0
- * must be zero), rank_bias [W][4], line_weights [C+1][15][W], line_bias [W], all 16-byte aligned; W = width <= 256, a
- * multiple of 4 (the reference: 256).  Rows and masks as in
+ * must be zero), rank_bias [W][4], line_weights [C+1][15][W], line_bias [W] and out, all 16-byte aligned (rows are
+ * stored as float4 / 4 x bfloat16); W = width <= 256, a multiple of 4 (the reference: 256).  Rows and masks as in
  * ddz_encode_state_actions; only the envs [env_begin, env_begin + env_count) are processed and row_base is subtracted from
  * their row numbers (chunking).  out_bf16 != 0: rows are written as bfloat16.  Form-B builds read the form-B nibbles. */
 int ddz_q_features(const void* state, int variant, const int32_t* offsets, const uint64_t* actions_u64,

@@ -1,7 +1,9 @@
 """numpy restatement of what ddz_q_features computes (TEST INFRASTRUCTURE): the first-layer features of the reference's
 NetComplicated family (net.py:65-139) from per-rank nibbles and the lookup tables of agent.q_tables, without ever building
-the [n, C+1, 15, 4] input.  tests/ checks it against the torch module on the CPU (so the table construction and the formulas
-are validated where there is no GPU) and the CUDA kernel against it on the GPU."""
+the [n, C+1, 15, 4] input.  tests/ checks it against the torch module's float64 convolutions on the CPU, for left-aligned
+rows and for form-B rows (test_consumer_contract.py, test_q_features_kernel.py), so the table construction and the formulas
+are validated where there is no GPU.  The CUDA kernel is checked against the torch module directly, on the GPU
+(test_q_features_kernel.py)."""
 import numpy as np
 
 LUT = np.zeros((16, 4))
@@ -28,9 +30,11 @@ def features(nibbles, scales, T, rank_bias, L, line_bias):
 
 
 def nibbles_of(x):
-    """float [n, C+1, 15, 4] thermometer rows (possibly scaled) -> (nibbles int [n, C+1, 15], scales [n, C+1])"""
+    """float [n, C+1, 15, 4] thermometer rows (possibly scaled) -> (nibbles int [n, C+1, 15], scales [n, C+1]); a row whose
+    ones are right-aligned (form B's probability planes: slot 0 empty, slot 3 set) gets 8 + count, its entry of LUT"""
     x = np.asarray(x, np.float64)
     nib = (x > 0).sum(-1)
+    nib = np.where((x[..., 0] == 0) & (x[..., 3] > 0), 8 + nib, nib)
     scale = x.max(axis=(-1, -2))
     scale[scale == 0] = 1.0
     return nib, scale
