@@ -308,7 +308,8 @@ struct StepArgs {
     uint64_t seed, env0; uint32_t stepno; int32_t rewards[3];
     const int8_t* perm; const int8_t* lord_pile; int pool_games;
     int8_t* r; uint8_t* done; int8_t* cat; float* reward;
-    long long prev_cap;   // capacity of `actions` (0 = unknown): a list cut off by an overflow is never read past it
+    long long prev_cap;   // capacity of `actions` (-1 = unknown, lists complete): a list cut off by an overflow is never read
+                          // past it; 0 is a capacity like any other (nothing stored: every live env sits the step out)
 };
 struct OutArgs {
     int32_t* offsets; uint64_t* actions_u64; float4* actions_f32; long long cap; float4* face;
@@ -406,7 +407,7 @@ __global__ void __launch_bounds__(kThreads, kMinCtasPerSm) k_env(void* state, St
                 // its visible part: `cnt` counts the entries that were stored.  An env whose list was dropped altogether
                 // sits this step out -- counted in stats[7], but NOT a sticky error: its next list may fit again.
                 const int base = prev_off, full = prev_end - prev_off;
-                const int cnt = a.prev_cap > 0 ? (int)max(0ll, min((long long)full, a.prev_cap - base)) : full;
+                const int cnt = a.prev_cap >= 0 ? (int)max(0ll, min((long long)full, a.prev_cap - base)) : full;
                 long long idx = -1;
                 if (a.mode == DDZ_CHOICE_INDEX) idx = (int32_t)(uint32_t)choice_raw;
                 else if (a.mode == DDZ_CHOICE_MOD) idx = cnt > 0 ? (long long)((uint32_t)choice_raw % (uint32_t)cnt) : -1;
@@ -1049,7 +1050,7 @@ __global__ void __launch_bounds__(kSearchWarps * 32) k_mcts_moves(const uint64_t
     if (lane == 0) counts[pair] = count;
 }
 
-// Batched dqn.py:50-71: per env, the index of the best-scoring legal move (first maximum, like torch.argmax), or with
+// Batched dqn.py:50-71: per env, the index of the best-scoring legal move (first maximum or first NaN, like torch.argmax), or with
 // probability epsilon a uniformly random one (e_greedy_action).  One lane per env; segments are short (mean 5.6).
 __global__ void __launch_bounds__(256) k_select_actions(const float* __restrict__ q, const int32_t* __restrict__ offsets,
                                                         float epsilon, uint64_t seed, uint64_t env0, uint32_t stepno,
@@ -1068,7 +1069,8 @@ __global__ void __launch_bounds__(256) k_select_actions(const float* __restrict_
         }
         if (!explore) {
             float bv = q[lo]; best = 0;
-            for (int i = 1; i < n; i++) { const float v = q[lo + i]; if (v > bv) { bv = v; best = i; } }
+            // the first NaN wins, as in torch.argmax: a NaN beats every number, and nothing beats a NaN
+            for (int i = 1; i < n; i++) { const float v = q[lo + i]; if (v > bv || (v != v && bv == bv)) { bv = v; best = i; } }
         }
     }
     choice[b] = best;
@@ -1251,6 +1253,7 @@ static int fill_step_args(StepArgs& a, const int32_t* offsets, const uint64_t* a
     for (int i = 0; i < 3; i++) a.rewards[i] = rewards ? rewards[i] : defR[i];
     a.r = r; a.done = done; a.cat = cat; a.reward = reward;
     a.pool_games = 1;
+    a.prev_cap = -1;   // ddz_step: complete lists (ddz_rollout_step sets the capacity)
     return 0;
 }
 
@@ -1273,7 +1276,8 @@ int ddz_rollout_step(void* state, void* workspace, int variant,
                      int32_t* out_offsets, uint64_t* out_actions_u64, float* out_actions_f32, int64_t cap,
                      float* face, int64_t* stats, int B, void* stream) {
     if (!state || !workspace || !out_offsets || !out_actions_u64 || B <= 0 || cap < 0) return DDZ_E_ARG;
-    if (out_offsets == prev_offsets || out_actions_u64 == prev_actions_u64) return DDZ_E_ARG;
+    // at cap = 0 nothing is read from or written to the action lists, so they may alias (ddz_rollout_steps' slices do)
+    if (out_offsets == prev_offsets || (cap > 0 && out_actions_u64 == prev_actions_u64)) return DDZ_E_ARG;
     if (face && ddz_face_channels(variant) < 0) return DDZ_E_ARG;
     if (perm && pool_games < 1) return DDZ_E_ARG;
     StepArgs a;

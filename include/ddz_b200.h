@@ -100,7 +100,8 @@ int ddz_reset(void* state, const int8_t* perm, const int8_t* lord_pile, int pool
  * Finished envs have no legal move.  If the total exceeds cap the tail is dropped and stats[7] is bumped; the offsets
  * are still those of the complete lists.  Nothing is read or written out of bounds and no env is lost: the fused step
  * plays a cut list from its visible part, an env whose list was dropped altogether sits that step out (stats[7] counts
- * it, no sticky error) and moves again as soon as a list of its own fits -- or observe again with a larger cap. */
+ * it, no sticky error) and moves again as soon as a list of its own fits -- or observe again with a larger cap.
+ * cap = 0 is valid: only the offsets (and the face) are written, and a fused step from such lists moves no env. */
 int ddz_observe(const void* state, void* workspace, int variant, int32_t* offsets, uint64_t* actions_u64,
                 float* actions_f32, int64_t cap, float* face, int64_t* stats, int B, void* stream);
 
@@ -123,8 +124,9 @@ int ddz_step(void* state, const int32_t* offsets, const uint64_t* actions_u64, c
 
 /* One fused env-step = ddz_step, then ddz_reset(only_done=1) when perm != NULL, then ddz_observe of the
  * new state, in ONE launch.  prev_* are the lists of the state being stepped, out_* receive the new
- * lists (ping-pong; they must not alias and both hold cap moves: of a list that an overflow cut off only the stored
- * part can be chosen from, never an out-of-bounds read). */
+ * lists (ping-pong; they must not alias -- the action lists may when cap = 0 -- and both hold cap moves: of a list that an
+ * overflow cut off only the stored part can be chosen from, never an out-of-bounds read; at cap = 0 every live env sits
+ * the step out). */
 int ddz_rollout_step(void* state, void* workspace, int variant,
                      const int32_t* prev_offsets, const uint64_t* prev_actions_u64,
                      const void* choice, int choice_mode, uint64_t seed, uint64_t env0, uint32_t stepno,
@@ -206,8 +208,9 @@ int ddz_encode_state_actions(const void* state, int variant, const int32_t* offs
                              const uint8_t* env_mask, const int32_t* dst_offsets, float* out, int B, void* stream);
 
 /* Batched DQNFirst.greedy_action / e_greedy_action (dqn.py:50-71): q float32[offsets[B]] are the Q-values the caller's
- * network gave to the legal moves (CSR order).  choice[b] = index of the first maximum of env b's segment (torch.argmax
- * semantics), or, with probability epsilon, a uniformly random index (Philox keyed by seed, env0+b, stepno); -1 for an
+ * network gave to the legal moves (CSR order).  choice[b] = index of the first maximum of env b's segment, or of its first
+ * NaN if it has one (torch.argmax semantics), or, with probability epsilon, a uniformly random index (Philox keyed by seed,
+ * env0+b, stepno); -1 for an
  * env without legal moves (finished).  Feed choice to ddz_step / ddz_rollout_step with DDZ_CHOICE_INDEX. */
 int ddz_select_actions(const float* q, const int32_t* offsets, float epsilon, uint64_t seed, uint64_t env0,
                        uint32_t stepno, int32_t* choice, int B, void* stream);

@@ -484,6 +484,7 @@ def test_select_actions_kernel(D, oracle):
     q = rng.standard_normal(off[-1]).astype(np.float32)
     q[rng.integers(0, len(q), 2000)] = 0.5          # ties: the FIRST maximum must win, like torch.argmax
     q[rng.integers(0, len(q), 2000)] = 3.0
+    q0, off0 = q, off
 
     class FakeEnv:
         pass
@@ -492,17 +493,70 @@ def test_select_actions_kernel(D, oracle):
     env.offsets = torch.as_tensor(off).cuda()
     pol = D.BatchedGreedyPolicy(None, epsilon=0.0, seed=9)
     got = pol.select(env, torch.as_tensor(q).cuda()).cpu().numpy()
-    want = np.array([np.argmax(q[off[b]:off[b + 1]]) if cnt[b] else -1 for b in range(B)])
-    assert np.array_equal(got, want)
+    assert np.array_equal(got, np.array([int(torch.argmax(torch.from_numpy(q[off[b]:off[b + 1]]))) if cnt[b] else -1
+                                         for b in range(B)]))
     pol = D.BatchedGreedyPolicy(None, epsilon=1.0, seed=9)
     got = pol.select(env, torch.as_tensor(q).cuda()).cpu().numpy()
     want = np.array([oracle.philox(9 ^ 0xD1B54A32D192ED03, 77 + b, 5) % cnt[b] if cnt[b] else -1 for b in range(B)])
     assert np.array_equal(got, want)
-    pol = D.BatchedGreedyPolicy(None, epsilon=0.3, seed=9)
-    got = pol.select(env, torch.as_tensor(q).cuda()).cpu().numpy()
-    greedy = np.array([np.argmax(q[off[b]:off[b + 1]]) if cnt[b] else -1 for b in range(B)])
-    frac = np.mean((got != greedy)[cnt > 1])
-    assert 0.15 < frac < 0.35                        # explores about 30 % of the time (minus lucky draws)
+    # the reference is torch.argmax per segment on the CPU, NaNs and infinities included; exploration is exact: env b
+    # explores iff float32(philox(seed ^ PHI, env0 + b, stepno) >> 8) * 2^-24 < float32(epsilon), then takes
+    # philox(seed ^ 0xD1B5..., ...) % n
+    def launch(q, off, eps, seed, env0, stepno):
+        B = len(off) - 1
+        out = torch.empty(B, dtype=torch.int32, device="cuda")
+        qd = torch.as_tensor(q if len(q) else np.zeros(1, np.float32)).cuda()
+        od = torch.as_tensor(off).cuda()
+        assert D.native.lib.ddz_select_actions(qd.data_ptr(), od.data_ptr(), eps, seed, env0, stepno, out.data_ptr(), B,
+                                               torch.cuda.current_stream().cuda_stream) == 0
+        return out.cpu().numpy()
+
+    def reference(q, off, eps, seed, env0, stepno):
+        qt, res = torch.from_numpy(q), []
+        e32 = np.float32(eps)
+        for b in range(len(off) - 1):
+            lo, hi = int(off[b]), int(off[b + 1])
+            if hi == lo:
+                res.append(-1)
+                continue
+            if e32 > 0:
+                u = oracle.philox(seed ^ 0x9E3779B97F4A7C15, env0 + b, stepno)
+                if np.float32(u >> 8) * np.float32(2.0 ** -24) < e32:
+                    res.append(oracle.philox(seed ^ 0xD1B54A32D192ED03, env0 + b, stepno) % (hi - lo))
+                    continue
+            res.append(int(torch.argmax(qt[lo:hi])))
+        return np.array(res)
+
+    nan, inf, tiny = np.float32(np.nan), np.float32(np.inf), np.float32(1e-45)
+    segs = [[nan, 1, 2], [1, nan, 3, nan], [1, 2, nan], [nan, nan], [5, nan, 7, nan, 9], [-inf, -inf, -inf], [-inf],
+            [1, inf, inf, 2], [-inf, inf], [nan, inf], [inf, nan], [-0.0, 0.0], [0.0, -0.0], [-0.0, -0.0, 0.0],
+            [tiny, 2 * tiny, 3 * tiny, 2 * tiny], [3 * tiny, tiny], [0.0, tiny, -tiny], [np.float32(-1e-38)] * 3, [7.0]]
+    segs.append(rng.standard_normal(512).astype(np.float32))               # DDZ_MAX_LEGAL moves
+    long_nan = rng.standard_normal(512).astype(np.float32)
+    long_nan[[300, 400]] = nan
+    segs.append(long_nan)
+    segs += [[], [nan]]
+    q = np.concatenate([np.asarray(s, np.float32) for s in segs]).astype(np.float32)
+    off = np.concatenate([[0], np.cumsum([len(s) for s in segs])]).astype(np.int32)
+    w = reference(q, off, 0.0, 9, 0, 0)
+    assert list(w[:4]) == [0, 1, 2, 0] and w[7] == 1 and w[11] == 0 and w[12] == 0   # torch: the first NaN / maximum
+    assert np.array_equal(launch(q, off, 0.0, 9, 0, 0), w)
+    for Bn in (1, 255, 257, 70000):                 # batch sizes around the 256-thread block, and many blocks
+        cnt = rng.integers(1, 12, Bn)
+        cnt[rng.random(Bn) < 0.05] = 0
+        o = np.concatenate([[0], np.cumsum(cnt)]).astype(np.int32)
+        qq = rng.standard_normal(int(o[-1])).astype(np.float32)
+        qq[rng.random(len(qq)) < 0.05] = nan
+        qq[rng.random(len(qq)) < 0.05] = inf
+        qq[rng.random(len(qq)) < 0.05] = -inf
+        assert np.array_equal(launch(qq, o, 0.0, 3, 5, 1), reference(qq, o, 0.0, 3, 5, 1)), Bn
+    # exact exploration on the edge segments and the first batch, with env0 past 2^32 too (a non-zero high word in the
+    # Philox counter); epsilon reaches the kernel as a C float (0.3 -> 0.30000001)
+    qe = np.concatenate([q, q0])
+    oe = np.concatenate([off[:-1], off0 + off[-1]]).astype(np.int32)
+    for eps in (1e-8, 0.01, 0.3, 0.5, float(np.nextafter(np.float32(1), np.float32(0)))):
+        for env0 in (77, (1 << 32) + 77):
+            assert np.array_equal(launch(qe, oe, eps, 9, env0, 5), reference(qe, oe, eps, 9, env0, 5)), (eps, env0)
 
 
 def test_dqn_lord_vs_random_matches_oracle_env(D, oracle):
