@@ -35,6 +35,7 @@
 #include "../../include/ddz_b200.h"
 #include "ddz_device.cuh"
 #include <cuda_bf16.h>
+#include <math_constants.h>
 #include "ddz_flat.cuh"
 #include "ddz_search.cuh"
 
@@ -953,6 +954,31 @@ struct KeySink {
     uint16_t* keys; int n, handnum;
     DDZ_DEV void operator()(uint64_t mv) { if (n < DDZ_MAX_LEGAL) keys[n] = (uint16_t)search::value_key(mv, handnum); n++; }
 };
+// one lane's playout of env e (Philox stream `env`, decisions stepno0, stepno0 + 1, ...): the body of k_playout, also
+// the default policy of k_uct
+template <bool PRUNED>
+DDZ_DEV void playout_env(Env& e, int max_steps, uint64_t seed, uint64_t env, uint32_t stepno0, const int32_t* rewards,
+                         int& steps, int& passes, int& over, int& winner) {
+    for (int t = 0; t < max_steps && !e.done(); t++) {
+        const uint64_t hand = hand_to_move(e), last = trick_of(e);
+        const Masks m = masks_of(hand);
+        const Rule ru = rule_of(last);
+        const int n = count_legal(m, ru, last != 0);
+        if (n <= 0) break;
+        const uint32_t u = philox(seed, env, stepno0 + (uint32_t)t);
+        int k;
+        if (PRUNED && n > search::kPruneAbove) {
+            uint16_t keys[DDZ_MAX_LEGAL];
+            KeySink ks{keys, 0, card_count(hand)};
+            enumerate_legal(m, ru, last != 0, ks);
+            const int nk = min(n, DDZ_MAX_LEGAL);            // 512 bounds every list of hands dealt from one deck
+            k = search::pruned_pick(keys, nk, (int)(u % (uint32_t)search::pruned_size(nk)));
+        } else k = (int)(u % (uint32_t)n);
+        const StepOut so = apply_move(e, select_legal(m, ru, last != 0, k), rewards);
+        steps++; passes += so.pass;
+        if (so.done) { over = 1; winner = so.winner; }
+    }
+}
 template <bool PRUNED>
 __global__ void __launch_bounds__(128) k_playout(void* state, int max_steps, uint64_t seed, uint64_t env0, uint32_t stepno0,
                                                  int32_t rw0, int32_t rw1, int32_t rw2, int32_t* __restrict__ steps_taken,
@@ -963,25 +989,7 @@ __global__ void __launch_bounds__(128) k_playout(void* state, int max_steps, uin
     if (b < B) {
         const StateView v = view_of(state, B);
         Env e = load_env(v, b);
-        for (int t = 0; t < max_steps && !e.done(); t++) {
-            const uint64_t hand = hand_to_move(e), last = trick_of(e);
-            const Masks m = masks_of(hand);
-            const Rule ru = rule_of(last);
-            const int n = count_legal(m, ru, last != 0);
-            if (n <= 0) break;
-            const uint32_t u = philox(seed, env0 + (uint64_t)b, stepno0 + (uint32_t)t);
-            int k;
-            if (PRUNED && n > search::kPruneAbove) {
-                uint16_t keys[DDZ_MAX_LEGAL];
-                KeySink ks{keys, 0, card_count(hand)};
-                enumerate_legal(m, ru, last != 0, ks);
-                const int nk = min(n, DDZ_MAX_LEGAL);            // 512 bounds every list of hands dealt from one deck
-                k = search::pruned_pick(keys, nk, (int)(u % (uint32_t)search::pruned_size(nk)));
-            } else k = (int)(u % (uint32_t)n);
-            const StepOut so = apply_move(e, select_legal(m, ru, last != 0, k), rewards);
-            steps++; passes += so.pass;
-            if (so.done) { over = 1; winner = so.winner; }
-        }
+        playout_env<PRUNED>(e, max_steps, seed, env0 + (uint64_t)b, stepno0, rewards, steps, passes, over, winner);
         store_env(v, b, e);
         if (steps_taken) steps_taken[b] = steps;
     }
@@ -1000,25 +1008,16 @@ struct SlotEmitter {
     uint64_t* out;
     DDZ_DEV void operator()(int idx, uint64_t mv) { if ((unsigned)idx < (unsigned)DDZ_MAX_LEGAL) out[idx] = mv; }
 };
-__global__ void __launch_bounds__(kSearchWarps * 32) k_mcts_moves(const uint64_t* __restrict__ hands,
-                                                                  const uint64_t* __restrict__ lasts,
-                                                                  uint64_t* __restrict__ out, int32_t* __restrict__ counts,
-                                                                  int npairs) {
+// The whole warp builds the pruned list of (hand, last) into dst[0 .. returned count): the full canonical list goes to
+// moves[0 .. nfull) and the keys to keys[] (per-warp scratch, DDZ_MAX_LEGAL entries each).  Shared by k_mcts_moves and k_uct.
+DDZ_DEV int warp_mcts_list(uint64_t hand, uint64_t last, uint64_t* moves, uint16_t* keys, uint64_t* dst, int lane, int& nfull) {
     constexpr unsigned FULL = 0xFFFFFFFFu;
-    __shared__ uint64_t s_moves[kSearchWarps][DDZ_MAX_LEGAL];
-    __shared__ uint16_t s_keys[kSearchWarps][DDZ_MAX_LEGAL];
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    const int pair = blockIdx.x * kSearchWarps + wib;
-    if (pair >= npairs) return;
-    const uint64_t hand = hands[pair], last = lasts[pair];
     const Masks hm = masks_of(hand);
     const Rule ru = rule_of(last);
-    uint64_t* moves = s_moves[wib];
-    uint16_t* keys = s_keys[wib];
     SlotEmitter em{moves};
     const int n = min(enumerate_legal_warp(hm, ru, last != 0, lane, em), DDZ_MAX_LEGAL);   // 512 bounds every real list
+    nfull = n;
     __syncwarp();
-    uint64_t* dst = out + (size_t)pair * DDZ_MCTS_MAX_MOVES;
     int count = n;
     if (n <= search::kPruneAbove) {
         for (int i = lane; i < n; i += 32) dst[i] = moves[i];
@@ -1047,7 +1046,291 @@ __global__ void __launch_bounds__(kSearchWarps * 32) k_mcts_moves(const uint64_t
             if (pos == 0) for (int k = m; k < rounds; k++) dst[2 * k + 1] = mv;
         }
     }
+    return count;
+}
+__global__ void __launch_bounds__(kSearchWarps * 32) k_mcts_moves(const uint64_t* __restrict__ hands,
+                                                                  const uint64_t* __restrict__ lasts,
+                                                                  uint64_t* __restrict__ out, int32_t* __restrict__ counts,
+                                                                  int npairs) {
+    __shared__ uint64_t s_moves[kSearchWarps][DDZ_MAX_LEGAL];
+    __shared__ uint16_t s_keys[kSearchWarps][DDZ_MAX_LEGAL];
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const int pair = blockIdx.x * kSearchWarps + wib;
+    if (pair >= npairs) return;
+    int nfull;
+    const int count = warp_mcts_list(hands[pair], lasts[pair], s_moves[wib], s_keys[wib],
+                                     out + (size_t)pair * DDZ_MCTS_MAX_MOVES, lane, nfull);
     if (lane == 0) counts[pair] = count;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Batched UCT search (the reference's search bot, server/mcts/interface.py:37-45, for B positions in ONE launch):
+// one warp per root, all `budget` iterations of  tree policy -> default policy -> back-up  inside the kernel.  The tree
+// lives in the caller's workspace (UctNode, layout in ddz_b200.h); a node's children are the nodes whose parent it is, in
+// node order = expansion order, all within [first_child, last_child].  A node's entries (its move list) are recomputed
+// when one of them is expanded: the full canonical list (select_legal, closed form), or the bot's pruned list built by the
+// warp (warp_mcts_list) when it has more than 10 moves.  Playouts are spread over the lanes (playout_env).
+// Draws: the j-th tree draw of root b is philox(seed, env0 + b, 0x80000000 + j); playout w of iteration it draws from
+// the stream ((env0 + b) * budget + it) * width + w at steps 0, 1, ...
+// ------------------------------------------------------------------------------------------------
+struct UctNode {
+    uint32_t untried[16];       // bit j: entry j of the node's list is not expanded yet
+    uint64_t hand[3], recent[3];
+    uint64_t move;              // the move that led here (root: 0)
+    int32_t parent, first_child, last_child, nchild;   // root: parent -1; no child: first = last = -1
+    int32_t visits, wins;
+    int16_t nentries, remaining;
+    int16_t index;              // index of `move` in the parent's canonical legal list (root: -1)
+    int8_t cur, winner;         // role to move; role that emptied its hand with `move`, or -1
+    int32_t pad[2];
+};
+static_assert(sizeof(UctNode) == DDZ_UCT_NODE_BYTES, "UctNode layout is documented in ddz_b200.h");
+constexpr int kUctWarps = 4;
+constexpr int kUctPlayoutSteps = 512;   // a game ends within 3 x 54 decisions
+__host__ __device__ inline size_t uct_header_bytes(int B) { return ((size_t)B * 4 + 255) / 256 * 256; }
+
+struct UctArgs {
+    const void* state; const uint8_t* mask; char* ws; const double* ln;
+    int budget, width, prune; double c; uint64_t seed, env0;
+    int32_t* choice; uint64_t* move; int32_t* root_n; uint64_t* root_moves; int32_t* root_visits; int32_t* root_wins;
+    int root_stride, B;
+};
+
+// entries of the list of the player to move: the canonical list, or its pruned form (same length rule as ddz_mcts_moves)
+DDZ_DEV int uct_entries(uint64_t hand, uint64_t last, int prune) {
+    const int n = count_legal(masks_of(hand), rule_of(last), last != 0);
+    return prune ? search::pruned_size(min(n, DDZ_MAX_LEGAL)) : n;
+}
+DDZ_DEV uint64_t uct_trick(const uint64_t* recent, int cur) {
+    return last_move(recent[(cur + 2) % 3], recent[(cur + 1) % 3]);
+}
+// node `id` with the given position; lane 0 writes the scalars, lanes 0..15 the untried bits
+DDZ_DEV void uct_init(UctNode* T, int id, const uint64_t* hand, const uint64_t* recent, int cur, int winner, uint64_t move,
+                      int parent, int index, int prune, int lane) {
+    UctNode& X = T[id];
+    const int ne = winner >= 0 ? 0 : uct_entries(hand[cur], uct_trick(recent, cur), prune);
+    if (lane < 16) {
+        const int lo = 32 * lane;
+        X.untried[lane] = ne >= lo + 32 ? 0xFFFFFFFFu : (ne > lo ? (1u << (ne - lo)) - 1u : 0u);
+    }
+    if (lane == 0) {
+        for (int q = 0; q < 3; q++) { X.hand[q] = hand[q]; X.recent[q] = recent[q]; }
+        X.move = move; X.parent = parent; X.first_child = X.last_child = -1; X.nchild = 0;
+        X.visits = X.wins = 0; X.nentries = (int16_t)ne; X.remaining = (int16_t)ne; X.index = (int16_t)index;
+        X.cur = (int8_t)cur; X.winner = (int8_t)winner; X.pad[0] = X.pad[1] = 0;
+    }
+}
+// UCB1 of a child, in double with correctly rounded operations and no contraction: the CPU port (Python's float, C with
+// -ffp-contract=off) computes the same bits, so both order every pair of children identically, near-ties included.
+// ln_n comes from a host table (C library log), because the device log is not correctly rounded.
+DDZ_DEV double uct_value(int wins, int visits, double c, double ln_n) {
+    const double v = (double)visits;
+    return __dadd_rn(__ddiv_rn((double)wins, v), __dmul_rn(c, __dsqrt_rn(__ddiv_rn(__dmul_rn(2.0, ln_n), v))));
+}
+// The child of x with the maximum (want_max) or minimum value, a uniformly drawn one of them among exact ties (in
+// expansion order); final = the answer's rule: wins / visits, maximum.  Lane-parallel over the child range.
+DDZ_DEV int uct_best_child(const UctNode* T, int x, bool want_max, bool final, double c, double ln_n, uint64_t seed,
+                           uint64_t env, uint32_t& j, int lane) {
+    constexpr unsigned FULL = 0xFFFFFFFFu;
+    const int f = T[x].first_child, l = T[x].last_child;
+    double best = want_max ? -CUDART_INF : CUDART_INF;
+    for (int k = f + lane; k <= l; k += 32) {
+        if (T[k].parent != x) continue;
+        const double v = final ? __ddiv_rn((double)T[k].wins, (double)T[k].visits) : uct_value(T[k].wins, T[k].visits, c, ln_n);
+        best = want_max ? fmax(best, v) : fmin(best, v);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double w = __shfl_xor_sync(FULL, best, o);
+        best = want_max ? fmax(best, w) : fmin(best, w);
+    }
+    int tied = 0;
+    for (int base = f; base <= l; base += 32) {
+        const int k = base + lane;
+        bool t = false;
+        if (k <= l && T[k].parent == x)
+            t = (final ? __ddiv_rn((double)T[k].wins, (double)T[k].visits) : uct_value(T[k].wins, T[k].visits, c, ln_n)) == best;
+        tied += __popc(__ballot_sync(FULL, t));
+    }
+    int r = 0;
+    if (tied >= 2) r = (int)(philox(seed, env, 0x80000000u + j++) % (uint32_t)tied);
+    for (int base = f; base <= l; base += 32) {
+        const int k = base + lane;
+        bool t = false;
+        if (k <= l && T[k].parent == x)
+            t = (final ? __ddiv_rn((double)T[k].wins, (double)T[k].visits) : uct_value(T[k].wins, T[k].visits, c, ln_n)) == best;
+        const unsigned bal = __ballot_sync(FULL, t);
+        if (r < __popc(bal)) return base + __fns(bal, 0, r + 1);
+        r -= __popc(bal);
+    }
+    return -1;   // not reached: x has at least one child
+}
+
+// One playout played by the whole warp, for width 1 with pruned lists (otherwise one lane plays while 31 wait): every lane
+// holds the same env, and a decision over a list of more than 10 moves takes entry u % count of the pruned list the warp
+// builds with warp_mcts_list -- the move k_playout<true>'s single lane finds with pruned_pick.  Returns the winner (-1: not
+// finished within kUctPlayoutSteps, which a game cannot reach).  Measured against the lane version in DESIGN.md 4; build
+// with -DDDZ_UCT_LANE_PLAYOUT for that version.
+DDZ_DEV int uct_warp_playout(Env e, uint64_t seed, uint64_t stream, uint64_t* moves, uint16_t* keys, uint64_t* list, int lane) {
+    const int32_t zero_rewards[3] = {0, 0, 0};
+    for (int t = 0; t < kUctPlayoutSteps && !e.done(); t++) {
+        const uint64_t hand = hand_to_move(e), last = trick_of(e);
+        const Masks m = masks_of(hand);
+        const Rule ru = rule_of(last);
+        const int n = count_legal(m, ru, last != 0);
+        if (n <= 0) break;
+        const uint32_t u = philox(seed, stream, (uint32_t)t);
+        uint64_t mv;
+        if (n > search::kPruneAbove) {
+            int nfull;
+            const int count = warp_mcts_list(hand, last, moves, keys, list, lane, nfull);
+            __syncwarp();
+            mv = list[u % (uint32_t)count];
+            __syncwarp();                         // every lane has read the list before the next decision rebuilds it
+        } else mv = select_legal(m, ru, last != 0, (int)(u % (uint32_t)n));
+        const StepOut so = apply_move(e, mv, zero_rewards);
+        if (so.done) return so.winner;
+    }
+    return -1;
+}
+
+__global__ void __launch_bounds__(kUctWarps * 32) k_uct(UctArgs a) {
+    constexpr unsigned FULL = 0xFFFFFFFFu;
+    __shared__ uint64_t s_moves[kUctWarps][DDZ_MAX_LEGAL];
+    __shared__ uint16_t s_keys[kUctWarps][DDZ_MAX_LEGAL];
+    __shared__ uint64_t s_list[kUctWarps][DDZ_MCTS_MAX_MOVES];
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const int b = blockIdx.x * kUctWarps + wib;
+    if (b >= a.B) return;
+    int32_t* nnodes = (int32_t*)a.ws + b;
+    UctNode* T = (UctNode*)(a.ws + uct_header_bytes(a.B)) + (size_t)b * (size_t)(a.budget + 1);
+    const Env e = load_env(view_of(const_cast<void*>(a.state), a.B), b);
+    const bool live = !(a.mask && !a.mask[b]) && !e.done() &&
+                      uct_entries(hand_to_move(e), trick_of(e), a.prune) > 0;
+    if (!live) {                                  // masked out, finished, or nothing to play: sentinels, no draws
+        if (lane == 0) {
+            a.choice[b] = -1;
+            if (a.move) a.move[b] = ~0ull;
+            if (a.root_n) a.root_n[b] = 0;
+            *nnodes = 0;
+        }
+        return;
+    }
+    const int me = e.cur();
+    const uint64_t env = a.env0 + (uint64_t)b;
+    const int32_t zero_rewards[3] = {0, 0, 0};
+    uint32_t j = 0;                               // tree draws taken so far
+    int nn = 1;
+    uct_init(T, 0, e.hand, e.recent, me, -1, 0ull, -1, -1, a.prune, lane);
+    __syncwarp();
+    for (int it = 0; it < a.budget; it++) {
+        // tree policy
+        int x = 0;
+        while (T[x].winner < 0) {
+            const UctNode& X = T[x];
+            const int remaining = X.remaining;
+            if (remaining > 0) {                  // expand the i-th remaining entry (list.pop(i)) and stop
+                const int i = (int)(philox(a.seed, env, 0x80000000u + j++) % (uint32_t)remaining);
+                const uint32_t w = lane < 16 ? X.untried[lane] : 0u;
+                const int pc = __popc(w);
+                int incl = pc;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(FULL, incl, o); if (lane >= o) incl += v; }
+                const bool mine = i >= incl - pc && i < incl;
+                const int wl = __ffs(__ballot_sync(FULL, mine)) - 1;
+                const int bit = mine ? (int)__fns(w, 0, i - (incl - pc) + 1) : 0;
+                const int entry = __shfl_sync(FULL, wl * 32 + bit, wl);
+                const int cur = X.cur;
+                uint64_t hand[3] = {X.hand[0], X.hand[1], X.hand[2]}, recent[3] = {X.recent[0], X.recent[1], X.recent[2]};
+                const uint64_t h = hand[cur], last = uct_trick(recent, cur);
+                const Masks m = masks_of(h);
+                const Rule ru = rule_of(last);
+                const int n = count_legal(m, ru, last != 0);
+                uint64_t mv;
+                int index;
+                if (a.prune && n > search::kPruneAbove) {
+                    int nfull;
+                    warp_mcts_list(h, last, s_moves[wib], s_keys[wib], s_list[wib], lane, nfull);
+                    __syncwarp();
+                    mv = s_list[wib][entry];
+                    int idx = DDZ_MAX_LEGAL;
+                    for (int k = lane; k < nfull; k += 32) if (s_moves[wib][k] == mv) idx = min(idx, k);
+                    index = __reduce_min_sync(FULL, idx);
+                    __syncwarp();
+                } else {
+                    mv = select_legal(m, ru, last != 0, entry);
+                    index = entry;
+                }
+                __syncwarp();                     // every lane has read X before it changes
+                if (lane == wl) T[x].untried[lane] = w & ~(1u << bit);
+                if (lane == 0) {
+                    T[x].remaining = (int16_t)(remaining - 1);
+                    if (T[x].first_child < 0) T[x].first_child = nn;
+                    T[x].last_child = nn;
+                    T[x].nchild += 1;
+                }
+                hand[cur] -= mv;
+                recent[cur] = mv;
+                const int winner = (mv != 0 && hand[cur] == 0) ? cur : -1;
+                uct_init(T, nn, hand, recent, (cur + 1) % 3, winner, mv, x, index, a.prune, lane);
+                __syncwarp();
+                x = nn++;
+                break;
+            }
+            x = uct_best_child(T, x, X.cur == me, false, a.c, a.ln[X.visits], a.seed, env, j, lane);
+        }
+        // default policy
+        int reward;
+        const UctNode& L = T[x];
+        if (L.winner >= 0) {
+            reward = ((L.winner == 1) == (me == 1)) ? a.width : 0;
+        }
+#ifndef DDZ_UCT_LANE_PLAYOUT
+        else if (a.prune && a.width == 1) {
+            Env pe;
+            for (int q = 0; q < 3; q++) { pe.hand[q] = L.hand[q]; pe.hist[q] = 0; pe.recent[q] = L.recent[q]; }
+            pe.meta = (uint32_t)L.cur;
+            const uint64_t stream = (a.env0 + (uint64_t)b) * (uint64_t)a.budget + (uint64_t)it;
+            const int winner = uct_warp_playout(pe, a.seed, stream, s_moves[wib], s_keys[wib], s_list[wib], lane);
+            reward = (winner >= 0 && ((winner == 1) == (me == 1))) ? 1 : 0;
+        }
+#endif
+        else {
+            int won = 0;
+            for (int w = lane; w < a.width; w += 32) {
+                Env pe;
+                for (int q = 0; q < 3; q++) { pe.hand[q] = L.hand[q]; pe.hist[q] = 0; pe.recent[q] = L.recent[q]; }
+                pe.meta = (uint32_t)L.cur;
+                int steps = 0, passes = 0, over = 0, winner = 0;
+                const uint64_t stream = ((a.env0 + (uint64_t)b) * (uint64_t)a.budget + (uint64_t)it) * (uint64_t)a.width + (uint64_t)w;
+                if (a.prune) playout_env<true>(pe, kUctPlayoutSteps, a.seed, stream, 0, zero_rewards, steps, passes, over, winner);
+                else playout_env<false>(pe, kUctPlayoutSteps, a.seed, stream, 0, zero_rewards, steps, passes, over, winner);
+                won += (over && ((winner == 1) == (me == 1))) ? 1 : 0;
+            }
+            reward = __reduce_add_sync(FULL, won);
+        }
+        // back-up
+        __syncwarp();
+        if (lane == 0)
+            for (int y = x; y >= 0; y = T[y].parent) { T[y].visits += a.width; T[y].wins += reward; }
+        __syncwarp();
+    }
+    // answer: the root child with the best wins / visits; the root's children are nodes 1 .. nchild (the first
+    // iterations expand the root until it is full)
+    const int best = uct_best_child(T, 0, true, true, 0.0, 0.0, a.seed, env, j, lane);
+    const int nroot = T[0].nchild;
+    if (a.root_n) {
+        for (int k = lane; k < min(nroot, a.root_stride); k += 32) {
+            const size_t o = (size_t)b * (size_t)a.root_stride + (size_t)k;
+            a.root_moves[o] = T[1 + k].move; a.root_visits[o] = T[1 + k].visits; a.root_wins[o] = T[1 + k].wins;
+        }
+    }
+    if (lane == 0) {
+        a.choice[b] = T[best].index;
+        if (a.move) a.move[b] = T[best].move;
+        if (a.root_n) a.root_n[b] = nroot;
+        *nnodes = nn;
+    }
 }
 
 // Batched dqn.py:50-71: per env, the index of the best-scoring legal move (first maximum or first NaN, like torch.argmax), or with
@@ -1727,6 +2010,29 @@ int ddz_mcts_moves(const uint64_t* hands, const uint64_t* lasts, uint64_t* moves
     k_mcts_moves<<<(n + kSearchWarps - 1) / kSearchWarps, kSearchWarps * 32, 0, (cudaStream_t)stream>>>(hands, lasts, moves,
                                                                                                         counts, n);
     DDZ_LAUNCH_CHECK("k_mcts_moves");
+    return 0;
+}
+
+size_t ddz_uct_workspace_bytes(int B, int budget) {
+    if (B <= 0 || budget < 1 || budget > DDZ_UCT_MAX_BUDGET) return 0;
+    return uct_header_bytes(B) + (size_t)B * (size_t)(budget + 1) * sizeof(UctNode);
+}
+
+int ddz_uct_search(const void* state, const uint8_t* env_mask, void* workspace, int budget, int width, int prune, double c,
+                   const double* ln_table, uint64_t seed, uint64_t env0, int32_t* choice, uint64_t* move,
+                   int32_t* root_n, uint64_t* root_moves, int32_t* root_visits, int32_t* root_wins, int root_stride,
+                   int B, void* stream) {
+    if (!state || !workspace || !ln_table || !choice || B <= 0) return DDZ_E_ARG;
+    if (budget < 1 || budget > DDZ_UCT_MAX_BUDGET || width < 1 || width > DDZ_UCT_MAX_WIDTH) return DDZ_E_ARG;
+    if ((int64_t)budget * width > DDZ_UCT_MAX_PLAYOUTS || !(c == c) || c - c != 0.0) return DDZ_E_ARG;   // c finite
+    if (root_n && (!root_moves || !root_visits || !root_wins || root_stride < 1)) return DDZ_E_ARG;
+    UctArgs a;
+    a.state = state; a.mask = env_mask; a.ws = (char*)workspace; a.ln = ln_table;
+    a.budget = budget; a.width = width; a.prune = prune != 0; a.c = c; a.seed = seed; a.env0 = env0;
+    a.choice = choice; a.move = move; a.root_n = root_n; a.root_moves = root_moves; a.root_visits = root_visits;
+    a.root_wins = root_wins; a.root_stride = root_stride; a.B = B;
+    k_uct<<<(B + kUctWarps - 1) / kUctWarps, kUctWarps * 32, 0, (cudaStream_t)stream>>>(a);
+    DDZ_LAUNCH_CHECK("k_uct");
     return 0;
 }
 

@@ -134,3 +134,25 @@ def mcts(payload, computation_budget=1000, seed=1, device=None, width=1, return_
     best = search.best_move()
     move = [r + 3 for r in range(15) for _ in range(int(best[r]))]
     return (move, search) if return_search else move
+
+
+def mcts_batch(payloads, computation_budget=1000, seed=1, width=1, prune=True, device=None):
+    """mcts(payload) for a whole list of payloads in ONE device launch (search.uct_search): the same full-information
+    payloads ({'role_id', 'hand_card': {role: [...]} for all three roles, 'last_taken'}), one search tree per payload, all
+    draws from Philox (so the answers are those of uct_search, not of the host-tree mcts()).  Returns one list of card
+    values per payload ([] = pass, or no move to make)."""
+    from .env import BatchedEnv
+    from .search import uct_search
+    get = lambda d, q: d[q] if q in d else d[str(q)]
+    role = np.array([int(p["role_id"]) for p in payloads], np.int64)
+    hands = np.stack([np.stack([_counts(get(p["hand_card"], q)) for q in range(3)]) for p in payloads])
+    last = np.stack([np.stack([_counts(get(p["last_taken"], q)) for q in range(3)]) for p in payloads])
+    B = len(payloads)
+    env = env_from_arrays(role, hands[np.arange(B), role], np.zeros((B, 3, 15), np.int64), last, hands.sum(2),
+                          env_cls=BatchedEnv, hands=hands, device=device)
+    choice, moves = uct_search(env, computation_budget=computation_budget, width=width, prune=prune, seed=seed)
+    out = []
+    for ch, mv in zip(choice.tolist(), moves.tolist()):
+        counts = [(mv >> (4 * r)) & 15 for r in range(15)] if ch >= 0 else [0] * 15
+        out.append([r + 3 for r in range(15) for _ in range(counts[r])])
+    return out

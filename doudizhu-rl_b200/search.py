@@ -37,6 +37,8 @@ from .deals import pack_counts_np
 from .env import BatchedEnv, MoveGenerator
 
 UCB_C = 0.7                      # get_bestchild.py:4
+_LN = {}                         # device -> ln table (float64, grown on demand)
+_WS = {}                         # (device, stream) -> search workspace (grown on demand, kept until release_workspaces())
 
 
 class _Node:
@@ -180,3 +182,80 @@ class UctSearch:
         counts int64 [15].  Consumes the generator when there is a tie: call it once."""
         moves, _, rate = self.root_table()
         return moves[self._pick(rate, rate.max())]
+
+
+# ---------------------------------------------------------------------------------------------------- batched search
+def _ln_table(n, device):
+    """float64 [>= n + 1] on `device`: ln_table[k] = math.log(k) (the C library's log, correctly rounded where the device's
+    is not; entry 0 is never read and holds 0)"""
+    t = _LN.get(device)
+    if t is None or t.numel() < n + 1:
+        t = torch.tensor([0.0] + [math.log(k) for k in range(1, n + 1)], dtype=torch.float64, device=device)
+        _LN[device] = t
+    return t
+
+
+def _workspace(nbytes, device, stream):
+    """the cached workspace of `stream`: one per stream, because a launch owns its workspace until it ends, so searches
+    on two concurrent streams must not share one"""
+    key = (device, stream)
+    t = _WS.get(key)
+    if t is None or t.numel() < nbytes:
+        _WS.pop(key, None)
+        t = torch.empty(max(nbytes, 8), dtype=torch.uint8, device=device)
+        _WS[key] = t
+    return t
+
+
+def release_workspaces():
+    """free the workspaces uct_search keeps for reuse: (B x (budget + 1) x 160 bytes each, e.g. 5.2 GB after a search
+    of 32 768 roots at budget 1000)"""
+    _WS.clear()
+
+
+def uct_search(env, computation_budget=1000, width=1, prune=True, c=UCB_C, seed=1, env_mask=None, root_table=False,
+               workspace=None):
+    """The search bot for every env of a BatchedEnv* in ONE launch (ddz_uct_search): root b is env b's position (all three
+    hands: full information), the searching player its role to move.  `computation_budget` iterations of the reference's
+    UCT (the same algorithm as UctSearch: UCB1 max for the searching player and min for the others, one expansion per
+    iteration, `width` random playouts of the expanded node, back-up, answer = root child with the best win rate), with
+    the bot's pruned move lists unless prune=False.  Every draw comes from Philox keyed by (seed, env.env0 + b), so a batch
+    split into chunks by env0 searches the same trees.  env_mask (bool [B]): only those envs are searched.
+    Returns (choice int32 [B], moves int64 [B]): the index of the chosen move in env.valid_actions() -- feed it to
+    env.step() -- and the packed move; -1 / ~0 for an env that is finished or masked out.  root_table=True adds
+    (root_n int32 [B], root_moves int64 [B,S], root_visits int32 [B,S], root_wins int32 [B,S]), the root's children in
+    expansion order (S = min(budget, 512)).  The env's state, step counter and lists are left as they are.
+    The search tree lives in a workspace of ddz_uct_workspace_bytes(B, budget) bytes: `workspace` (a device uint8 tensor
+    of at least that size, owned by the caller) or, by default, one cached per stream and kept for the next call (free
+    the cache with release_workspaces())."""
+    budget, width = int(computation_budget), int(width)
+    if not (1 <= budget <= N.UCT_MAX_BUDGET and 1 <= width <= N.UCT_MAX_WIDTH and budget * width <= N.UCT_MAX_PLAYOUTS):
+        raise ValueError("need 1 <= budget <= %d, 1 <= width <= %d and budget * width <= %d"
+                         % (N.UCT_MAX_BUDGET, N.UCT_MAX_WIDTH, N.UCT_MAX_PLAYOUTS))
+    B, dev = env.B, env.device
+    with torch.cuda.device(dev):
+        ln = _ln_table(budget * width, dev)
+        stream = torch.cuda.current_stream(dev)
+        need = N.lib.ddz_uct_workspace_bytes(B, budget)
+        if workspace is None:
+            ws = _workspace(need, dev, stream.cuda_stream)
+        else:
+            ws = workspace
+            if ws.device != dev or ws.dtype != torch.uint8 or not ws.is_contiguous() or ws.numel() < need:
+                raise ValueError("workspace must be a contiguous uint8 tensor of at least %d bytes on %s" % (need, dev))
+        mask = None if env_mask is None else torch.as_tensor(env_mask).to(dev, torch.bool).to(torch.uint8).contiguous()
+        if mask is not None and mask.numel() != B:
+            raise ValueError("env_mask must have B entries")
+        choice = torch.empty(B, dtype=torch.int32, device=dev)
+        moves = torch.empty(B, dtype=torch.int64, device=dev)
+        S = min(budget, N.MAX_LEGAL)
+        tab = None
+        if root_table:
+            tab = (torch.zeros(B, dtype=torch.int32, device=dev), torch.zeros((B, S), dtype=torch.int64, device=dev),
+                   torch.zeros((B, S), dtype=torch.int32, device=dev), torch.zeros((B, S), dtype=torch.int32, device=dev))
+        p = lambda t: None if t is None else t.data_ptr()
+        N.check(N.lib.ddz_uct_search(p(env._state), p(mask), ws.data_ptr(), budget, width, int(bool(prune)), float(c),
+                                     ln.data_ptr(), int(seed), env.env0, choice.data_ptr(), moves.data_ptr(),
+                                     *(p(t) for t in (tab or (None,) * 4)), S if root_table else 0, B,
+                                     stream.cuda_stream), "ddz_uct_search")
+    return (choice, moves) + ((tab,) if root_table else ())

@@ -42,7 +42,8 @@
 extern "C" {
 #endif
 
-#define DDZ_ABI_VERSION 3   /* 3: ddz_mcts_moves, ddz_playout_pruned, ddz_q_features.  2: ddz_mpipe_*, ddz_set_tile_order, ddz_prob_form; cut lists are played
+#define DDZ_ABI_VERSION 3   /* 3: ddz_mcts_moves, ddz_playout_pruned, ddz_q_features (+ ddz_uct_search, ddz_uct_workspace_bytes:
+                            * new entry points only, backward compatible).  2: ddz_mpipe_*, ddz_set_tile_order, ddz_prob_form; cut lists are played
                             * from their visible part */
 #define DDZ_MAX_LEGAL 512  /* upper bound of legal moves of one decision (worst known hand: 497) */
 
@@ -195,6 +196,48 @@ int ddz_q_features(const void* state, int variant, const int32_t* offsets, const
 int ddz_mcts_moves(const uint64_t* hands, const uint64_t* lasts, uint64_t* moves, int32_t* counts, int n, void* stream);
 int ddz_playout_pruned(void* state, int max_steps, uint64_t seed, uint64_t env0, uint32_t stepno0, const int32_t rewards[3],
                        int32_t* steps_taken, int64_t* stats, int B, void* stream);
+
+/* The search bot itself (server/mcts/interface.py:37-45) for B positions in ONE launch: `budget` iterations of UCT
+ * (tree policy: walk down while a node is fully expanded by UCB1 -- the maximum where the node's player is the searching
+ * player, the minimum elsewhere, partner farmer included --, expand one untried entry at the first node that has one;
+ * default policy: `width` random playouts to the end, = ddz_playout_pruned / ddz_playout, or width x won for a node whose
+ * move ended the game; back-up: visits += width, wins += playouts the searching side won), then the root child with the
+ * best wins / visits.  Root b is env b of `state` (read only): the searching player is the role to move, the trick to
+ * beat the previous hand-out (else the one before), hist is not used.  A node's entries are the bot's pruned list
+ * (ddz_mcts_moves order, duplicates are separate entries) when prune != 0, else the canonical list; the expanded entry is
+ * the i-th REMAINING untried entry in list order (list.pop(i)).
+ * Draws (Philox, as ddz_playout):
+ *   tree draw j of root b = philox(seed, env0 + b, 0x80000000 + j): j counts every expansion draw (u % remaining, taken even
+ *   when one entry remains) and every tie draw among k >= 2 exactly equal UCB / final values (u % k over the tied
+ *   children in expansion order), in the order they happen;
+ *   playout w of iteration it of root b = philox(seed, ((env0 + b) * budget + it) * width + w, t) at its decision t.
+ * UCB1 = wins / visits + c * sqrt(2 * ln_table[visits of the parent] / visits) in double, correctly rounded operations,
+ * no contraction; ln_table is device double[budget * width + 1], ln_table[n] = log((double)n) of the host C library.
+ * Outputs: choice int32[B] = index of the chosen move in the env's canonical legal list (feeds ddz_step /
+ * ddz_rollout_step with DDZ_CHOICE_INDEX), -1 for an env that is masked out (env_mask uint8[B] or NULL = all), finished or
+ * without a move; move uint64[B] (optional) = the packed move, or ~0.  Root table (optional; root_n NULL skips it):
+ * root_n int32[B] = number of root children, and for the first min(root_n, root_stride) of them in expansion order
+ * root_moves uint64 / root_visits int32 / root_wins int32 [B][root_stride].  Masked-out and finished roots take no draw,
+ * so they never shift another root's search; env0 chunks a batch (two calls over halves with their env0 = one call).
+ * Bounds: 1 <= budget <= DDZ_UCT_MAX_BUDGET, 1 <= width <= DDZ_UCT_MAX_WIDTH, budget * width <= DDZ_UCT_MAX_PLAYOUTS, c
+ * finite; else (or NULL state / workspace / ln_table / choice, B <= 0) DDZ_E_ARG before any CUDA call.
+ * Workspace (no zero-fill needed; one per concurrent launch), ddz_uct_workspace_bytes(B, budget) =
+ *   round_up(4 B, 256) + B (budget + 1) DDZ_UCT_NODE_BYTES  (0 for arguments out of range): int32 nnodes[B] (0 for a root
+ * that was not searched), then from byte round_up(4 B, 256) the tree of root b at node b * (budget + 1): node 0 is the
+ * root, node k the k-th one created (expansion order); a node's children are the nodes whose parent it is.  Node, 160 bytes:
+ *   0 uint32 untried[16] (bit j: entry j not expanded)   64 uint64 hand[3]   88 uint64 recent[3]
+ *   112 uint64 move (root 0)   120 int32 parent (root -1)   124 int32 first_child   128 int32 last_child (-1 / -1: none)
+ *   132 int32 nchild   136 int32 visits   140 int32 wins   144 int16 nentries   146 int16 remaining
+ *   148 int16 index (of move in the parent's canonical list; root -1)   150 int8 cur   151 int8 winner (-1: none)   152 pad */
+#define DDZ_UCT_MAX_BUDGET 65536
+#define DDZ_UCT_MAX_WIDTH 1024
+#define DDZ_UCT_MAX_PLAYOUTS (1 << 24)   /* budget * width */
+#define DDZ_UCT_NODE_BYTES 160
+size_t ddz_uct_workspace_bytes(int B, int budget);
+int ddz_uct_search(const void* state, const uint8_t* env_mask, void* workspace, int budget, int width, int prune, double c,
+                   const double* ln_table, uint64_t seed, uint64_t env0, int32_t* choice, uint64_t* move,
+                   int32_t* root_n, uint64_t* root_moves, int32_t* root_visits, int32_t* root_wins, int root_stride,
+                   int B, void* stream);
 
 /* Env.batch_arr2onehot over packed moves (envi.py:113,140-146): out float32[n][15][4] */
 int ddz_encode_actions(const uint64_t* actions_u64, int64_t n, float* out, void* stream);
