@@ -26,7 +26,8 @@ EXPORTS = ("ddz_abi_version", "ddz_prob_form", "ddz_set_tile_order", "ddz_face_c
            "ddz_encode_face", "ddz_select_actions", "ddz_kth_moves", "ddz_playout", "ddz_pipe_create", "ddz_pipe_destroy",
            "ddz_pipe_step", "ddz_pipe_wait", "ddz_pipe_refill", "ddz_pipe_flush", "ddz_rollout_steps", "ddz_encode_state_actions", "ddz_legal_count", "ddz_legal_emit", "ddz_rows_alloc", "ddz_rows_free",
            "ddz_mpipe_create", "ddz_mpipe_destroy", "ddz_mpipe_step", "ddz_mpipe_wait", "ddz_mpipe_refill", "ddz_mpipe_flush", "ddz_mpipe_join",
-           "ddz_mcts_moves", "ddz_playout_pruned", "ddz_q_features", "ddz_uct_workspace_bytes", "ddz_uct_search")
+           "ddz_mcts_moves", "ddz_playout_pruned", "ddz_q_features", "ddz_uct_workspace_bytes", "ddz_uct_search",
+           "ddz_determinize", "ddz_uct_pool")
 
 lib = C.CDLL(LIB_PATH)
 _missing = [name for name in EXPORTS if not hasattr(lib, name)]
@@ -75,6 +76,9 @@ lib.ddz_uct_workspace_bytes.argtypes = [_i, _i]
 lib.ddz_uct_workspace_bytes.restype = C.c_size_t
 lib.ddz_uct_search.argtypes = [_vp, _vp, _vp, _i, _i, _i, C.c_double, _vp, _u64, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp]
 UCT_MAX_BUDGET, UCT_MAX_WIDTH, UCT_MAX_PLAYOUTS, UCT_NODE_BYTES = 65536, 1024, 1 << 24, 160
+lib.ddz_determinize.argtypes = [_vp, _vp, _i, _u64, _u64, _vp, _vp, _i, _vp]
+lib.ddz_uct_pool.argtypes = [_vp, _i, _i, _vp, _vp, _vp, _vp, _i, _vp]
+PIMC_MAX_DETERMINIZATIONS = 4096
 lib.ddz_q_features.argtypes = [_vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i64, _vp, _vp, _vp, _vp, _i, _vp, _i, _i, _vp]
 lib.ddz_pipe_create.restype = _vp
 lib.ddz_pipe_destroy.argtypes = [_vp]

@@ -25,6 +25,7 @@
 // needs is many independent warps with stores in flight and no synchronisation.
 #include <cuda.h>
 #include <cuda_runtime.h>
+#include <climits>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -1333,6 +1334,113 @@ __global__ void __launch_bounds__(kUctWarps * 32) k_uct(UctArgs a) {
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Determinized search (PIMC): D full-information deals per root that agree with what the player to move has seen, searched
+// by k_uct as B * D trees, their root statistics added up per canonical list index (the root list depends only on the
+// mover's hand and the trick, so it is the same list in every determinization).
+// ------------------------------------------------------------------------------------------------
+constexpr uint32_t kDeterminizeStep = 0xC0000000u;   // Philox step of draw 0; k_uct's tree draws start at 0x80000000
+constexpr int kPoolWarps = 4;
+
+// One thread per output env i = b * D + d.  Unseen cards = deck - hand[m] - hist[0..2], walked in rank order; card j goes
+// to role a = (m+1)%3 with probability ra / (ra + rc) of the slots still open (selection sampling), else to c = (m+2)%3.
+__global__ void __launch_bounds__(256) k_determinize(const void* state, const uint8_t* __restrict__ mask, int D, uint64_t seed,
+                                                     uint64_t env0, void* out, int64_t* __restrict__ stats, int B) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)B * D) return;
+    const int b = (int)(i / D), d = (int)(i % D);
+    Env e = load_env(view_of(const_cast<void*>(state), B), b);
+    if (!(mask && !mask[b]) && !e.done()) {
+        const int m = e.cur(), a = (m + 1) % 3, c = (m + 2) % 3;
+        const uint64_t own = pick3(m, e.hand[0], e.hand[1], e.hand[2]);
+        const uint64_t ha = pick3(a, e.hand[0], e.hand[1], e.hand[2]), hc = pick3(c, e.hand[0], e.hand[1], e.hand[2]);
+        int ra = card_count(ha), rc = card_count(hc), unseen = 0;
+        bool bad = false;
+        uint64_t un = 0;
+        for (int r = 0; r < 15; r++) {
+            const int u = (r < 13 ? 4 : 1) - (int)((own >> (4 * r)) & 15) - (int)((e.hist[0] >> (4 * r)) & 15) -
+                          (int)((e.hist[1] >> (4 * r)) & 15) - (int)((e.hist[2] >> (4 * r)) & 15);
+            bad |= u < 0;
+            unseen += u;
+            if (u > 0) un |= (uint64_t)u << (4 * r);
+        }
+        if (bad || unseen != ra + rc) {           // no deal agrees with this view: finished with a sticky error
+            e.meta |= 4u | 32u;
+            if (d == 0 && stats) atomicAdd((unsigned long long*)&stats[7], 1ull);
+        } else {
+            const uint64_t ctr = (env0 + (uint64_t)b) * (uint64_t)D + (uint64_t)d;
+            uint64_t na = 0, nc = 0;
+            uint32_t j = 0;
+            for (int r = 0; r < 15; r++)
+                for (int k = (int)((un >> (4 * r)) & 15); k > 0; k--) {
+                    const uint32_t u = philox(seed, ctr, kDeterminizeStep + j++);
+                    if ((int)(u % (uint32_t)(ra + rc)) < ra) { na += 1ull << (4 * r); ra--; }
+                    else { nc += 1ull << (4 * r); rc--; }
+                }
+#pragma unroll
+            for (int q = 0; q < 3; q++) e.hand[q] = q == a ? na : (q == c ? nc : e.hand[q]);
+        }
+    }
+    store_env(view_of(out, B * D), (int)i, e);
+}
+
+// One warp per root b: the root children of trees b * D .. b * D + D - 1 (nodes first_child .. last_child whose parent is
+// 0) add their visits and wins into shared counters keyed by canonical index; then the index with the best pooled
+// wins / visits (exact 64-bit cross products, lowest index on ties).
+__global__ void __launch_bounds__(kPoolWarps * 32) k_uct_pool(const char* __restrict__ ws, int budget, int D, int32_t* choice,
+                                                              uint64_t* move, int32_t* pooled_visits, int32_t* pooled_wins, int B) {
+    constexpr unsigned FULL = 0xFFFFFFFFu;
+    __shared__ int32_t s_v[kPoolWarps][DDZ_MAX_LEGAL], s_w[kPoolWarps][DDZ_MAX_LEGAL];
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const int b = blockIdx.x * kPoolWarps + wib;
+    if (b >= B) return;
+    const int ntrees = B * D;
+    const int32_t* nnodes = (const int32_t*)ws;
+    const UctNode* base = (const UctNode*)(ws + uct_header_bytes(ntrees));
+    for (int k = lane; k < DDZ_MAX_LEGAL; k += 32) { s_v[wib][k] = 0; s_w[wib][k] = 0; }
+    __syncwarp();
+    int root = -1;                                // the first tree of b that was searched
+    for (int d = 0; d < D; d++) {
+        const int t = b * D + d;
+        if (nnodes[t] <= 0) continue;
+        if (root < 0) root = t;
+        const UctNode* T = base + (size_t)t * (size_t)(budget + 1);
+        const int f = T[0].first_child, l = T[0].last_child;
+        for (int k = f + lane; k >= 0 && k <= l; k += 32) {
+            if (T[k].parent != 0) continue;
+            const int idx = T[k].index;
+            if ((unsigned)idx >= (unsigned)DDZ_MAX_LEGAL) continue;
+            atomicAdd(&s_v[wib][idx], T[k].visits);
+            atomicAdd(&s_w[wib][idx], T[k].wins);
+        }
+    }
+    __syncwarp();
+    int bi = -1;
+    long long bv = 0, bw = 0;
+    for (int k = lane; k < DDZ_MAX_LEGAL; k += 32) {
+        const long long v = s_v[wib][k], w = s_w[wib][k];
+        if (pooled_visits) pooled_visits[(size_t)b * DDZ_MAX_LEGAL + k] = (int32_t)v;
+        if (pooled_wins) pooled_wins[(size_t)b * DDZ_MAX_LEGAL + k] = (int32_t)w;
+        if (v > 0 && (bi < 0 || w * bv > bw * v)) { bi = k; bv = v; bw = w; }   // ascending k: ties keep the lower index
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const int oi = __shfl_xor_sync(FULL, bi, o);
+        const long long ov = __shfl_xor_sync(FULL, bv, o), ow = __shfl_xor_sync(FULL, bw, o);
+        if (oi >= 0 && (bi < 0 || ow * bv > bw * ov || (ow * bv == bw * ov && oi < bi))) { bi = oi; bv = ov; bw = ow; }
+    }
+    if (lane == 0) {
+        uint64_t mv = ~0ull;
+        if (root >= 0 && bi >= 0) {
+            const UctNode& R = base[(size_t)root * (size_t)(budget + 1)];
+            const uint64_t last = uct_trick(R.recent, R.cur);
+            mv = select_legal(masks_of(R.hand[R.cur]), rule_of(last), last != 0, bi);
+        }
+        choice[b] = root >= 0 ? bi : -1;
+        if (move) move[b] = root >= 0 ? mv : ~0ull;
+    }
+}
+
 // Batched dqn.py:50-71: per env, the index of the best-scoring legal move (first maximum or first NaN, like torch.argmax), or with
 // probability epsilon a uniformly random one (e_greedy_action).  One lane per env; segments are short (mean 5.6).
 __global__ void __launch_bounds__(256) k_select_actions(const float* __restrict__ q, const int32_t* __restrict__ offsets,
@@ -2033,6 +2141,28 @@ int ddz_uct_search(const void* state, const uint8_t* env_mask, void* workspace, 
     a.root_wins = root_wins; a.root_stride = root_stride; a.B = B;
     k_uct<<<(B + kUctWarps - 1) / kUctWarps, kUctWarps * 32, 0, (cudaStream_t)stream>>>(a);
     DDZ_LAUNCH_CHECK("k_uct");
+    return 0;
+}
+
+int ddz_determinize(const void* state, const uint8_t* env_mask, int D, uint64_t seed, uint64_t env0, void* out_state,
+                    int64_t* stats, int B, void* stream) {
+    if (!state || !out_state || B <= 0 || D < 1 || D > DDZ_PIMC_MAX_DETERMINIZATIONS) return DDZ_E_ARG;
+    const long long n = (long long)B * D;
+    if (n > INT_MAX) return DDZ_E_ARG;
+    k_determinize<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(state, env_mask, D, seed, env0, out_state,
+                                                                                 stats, B);
+    DDZ_LAUNCH_CHECK("k_determinize");
+    return 0;
+}
+
+int ddz_uct_pool(const void* workspace, int budget, int D, int32_t* choice, uint64_t* move, int32_t* pooled_visits,
+                 int32_t* pooled_wins, int B, void* stream) {
+    if (!workspace || !choice || B <= 0 || budget < 1 || budget > DDZ_UCT_MAX_BUDGET) return DDZ_E_ARG;
+    if (D < 1 || D > DDZ_PIMC_MAX_DETERMINIZATIONS || (long long)B * D > INT_MAX || (long long)D * budget > INT_MAX)
+        return DDZ_E_ARG;
+    k_uct_pool<<<(B + kPoolWarps - 1) / kPoolWarps, kPoolWarps * 32, 0, (cudaStream_t)stream>>>(
+        (const char*)workspace, budget, D, choice, move, pooled_visits, pooled_wins, B);
+    DDZ_LAUNCH_CHECK("k_uct_pool");
     return 0;
 }
 

@@ -94,16 +94,27 @@ class BatchedDQN:
 class BatchedGame:
     """game.py:10-238 over a batched env.  nets_dict / dqns_dict / reward_dict / train_dict / preload keep the
     reference's meaning (role -> net class / DQN class / terminal reward magnitude / keep training / checkpoint path);
-    `dqns_dict[role]` is called as `dqn_cls(net_cls, face_channels, device)` (BatchedDQN's signature)."""
+    `dqns_dict[role]` is called as `dqn_cls(net_cls, face_channels, device)` (BatchedDQN's signature).
+    search_dict (optional) seats the search bot: role -> keyword arguments of search.pimc_search, e.g.
+    {"lord": {"determinizations": 8, "computation_budget": 125}}; that role plays from its own view (determinized UCT),
+    or with "determinizations": 0 the full-information search.uct_search, which sees every hand.  A role has a net or a
+    search entry, not both."""
 
     def __init__(self, env_cls, nets_dict, dqns_dict, reward_dict=None, train_dict=None, preload=None, seed=None,
-                 debug=False, num_envs=4096, pool_games=8, deals=None, device=None, updates_per_step=1):
+                 debug=False, num_envs=4096, pool_games=8, deals=None, device=None, updates_per_step=1, search_dict=None):
         if reward_dict is None:
             reward_dict = {"lord": 100, "down": 50, "up": 50}
         if train_dict is None:
             train_dict = {"lord": True, "down": True, "up": True}
         preload = preload or {}
         assert not (nets_dict.keys() ^ dqns_dict.keys()), "Net and DQN must match"
+        self.search_dict = {r: dict(kw) for r, kw in (search_dict or {}).items()}
+        for role in self.search_dict:
+            if role not in ROLE_INDEX:
+                raise ValueError("unknown role %r in search_dict" % (role,))
+            if nets_dict.get(role):
+                raise ValueError("role %r has both a net and a search entry" % (role,))
+        self._search_seed = int(seed) if seed else 0
         self.env = env_cls(num_envs, debug=debug, seed=seed, device=device)
         self.B, self.device = self.env.B, self.env.device
         self.reward_dict, self.train_dict, self.preload = reward_dict, train_dict, preload
@@ -195,6 +206,10 @@ class BatchedGame:
                 a0 = acts[(off[:-1] + k.clamp(min=0)).clamp(max=last)] * keep
                 a1 = acts[(off[:-1] + kg).clamp(max=last)] * keep
                 pending.append((role, self._collectors[role].on_turn(a0, a1)))
+        for role, kw in self.search_dict.items():
+            mine = (seat == ROLE_INDEX[role]) & live
+            if bool(mine.any()):
+                choice = torch.where(mine, self._search(kw, mine).to(torch.int64).clamp(min=0), choice)
         was_done = env.is_done.clone()
         env.step(choice.to(torch.int32))
         env.observe()
@@ -218,6 +233,17 @@ class BatchedGame:
         self.episodes += ended
         self.iterations += 1
         return ended
+
+    def _search(self, kw, mine):
+        """the search seat's choice for the envs of `mine`: pimc_search, or uct_search for determinizations = 0; the seed is
+        derived from (seed, iterations), so every decision draws afresh and a run is reproducible"""
+        from .search import pimc_search, uct_search
+        kw = dict(kw)
+        D = int(kw.pop("determinizations", 16))
+        seed = (self._search_seed * 1000003 + self.iterations + 1) & (2 ** 64 - 1)
+        if D == 0:
+            return uct_search(self.env, seed=seed, env_mask=mine, **kw)[0]
+        return pimc_search(self.env, determinizations=D, seed=seed, env_mask=mine, **kw)[0]
 
     def play(self, games=None):
         """decisions until `games` more games have ended (default: one per env, the batched `Game.play`)"""
@@ -268,13 +294,14 @@ class BatchedGame:
     # ------------------------------------------------------------------ evaluation (game.py:240-275)
     @staticmethod
     def compete(env_cls, nets_dict, dqns_dict, model_dict, total=1000, print_every=100, debug=True, num_envs=4096,
-                seed=None, device=None, nets=None):
+                seed=None, device=None, nets=None, search_dict=None):
         """greedy play of the given networks (others random) until `total` games have ended; Counter of wins per role.
-        `nets` may hand over already constructed networks per role instead of checkpoints in model_dict."""
+        `nets` may hand over already constructed networks per role instead of checkpoints in model_dict; search_dict
+        seats the search bot as in BatchedGame."""
         assert not (nets_dict.keys() ^ dqns_dict.keys()), "Net and DQN must match"
         train_dict = {r: False for r in ROLES}
         game = BatchedGame(env_cls, nets_dict, dqns_dict, train_dict=train_dict, preload=model_dict or {}, seed=seed,
-                           debug=False, num_envs=num_envs, device=device)
+                           debug=False, num_envs=num_envs, device=device, search_dict=search_dict)
         for role, net in (nets or {}).items():
             getattr(game, role).policy_net.load_state_dict(net.state_dict())
         wins = collections.Counter()

@@ -156,3 +156,36 @@ def mcts_batch(payloads, computation_budget=1000, seed=1, width=1, prune=True, d
         counts = [(mv >> (4 * r)) & 15 for r in range(15)] if ch >= 0 else [0] * 15
         out.append([r + 3 for r in range(15) for _ in range(counts[r])])
     return out
+
+
+def unseen_mismatch(role, hand, hist, left):
+    """indices of the positions whose unseen cards (full deck - own hand - everything played) cannot be the other two
+    hands: a rank seen more often than the deck holds it, or an unseen count other than the sum of their `left` sizes"""
+    role, hand, hist, left = (np.asarray(x, np.int64) for x in (role, hand, hist, left))
+    deck = np.array([4] * 13 + [1, 1], np.int64)
+    unseen = deck - hand - hist.sum(1)
+    B = len(role)
+    others = left[np.arange(B), (role + 1) % 3] + left[np.arange(B), (role + 2) % 3]
+    return np.flatnonzero((unseen < 0).any(1) | (unseen.sum(1) != others))
+
+
+def pimc_batch(payloads, determinizations=16, computation_budget=1000, seed=1, width=1, prune=True, device=None):
+    """The search bot for a list of payloads in the web bot's wire format ({'role_id', 'cur_cards', 'history',
+    'last_taken', 'left'}, server/client.py): the player sees only its own hand, so every payload is searched from that
+    view (search.pimc_search: `determinizations` deals of the unseen cards, one UCT tree each, root statistics pooled).
+    Returns one list of card values per payload ([] = pass), in the form mcts_batch uses.  Raises ValueError naming the
+    payloads whose unseen cards do not match the other players' `left` counts."""
+    from .env import BatchedEnv
+    from .search import pimc_search
+    role, hand, hist, last, left = payload_arrays(payloads)
+    bad = unseen_mismatch(role, hand, hist, left)
+    if len(bad):
+        raise ValueError("payloads %s: the unseen cards do not match the other players' `left` counts" % bad.tolist())
+    env = env_from_arrays(role, hand, hist, last, left, env_cls=BatchedEnv, device=device)
+    choice, moves = pimc_search(env, determinizations=determinizations, computation_budget=computation_budget, width=width,
+                                prune=prune, seed=seed)
+    out = []
+    for ch, mv in zip(choice.tolist(), moves.tolist()):
+        counts = [(mv >> (4 * r)) & 15 for r in range(15)] if ch >= 0 else [0] * 15
+        out.append([r + 3 for r in range(15) for _ in range(counts[r])])
+    return out

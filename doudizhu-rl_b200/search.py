@@ -213,6 +213,27 @@ def release_workspaces():
     _WS.clear()
 
 
+def _check_budget(computation_budget, width):
+    """(budget, width) as ints, or ValueError outside ddz_uct_search's bounds"""
+    budget, width = int(computation_budget), int(width)
+    if not (1 <= budget <= N.UCT_MAX_BUDGET and 1 <= width <= N.UCT_MAX_WIDTH and budget * width <= N.UCT_MAX_PLAYOUTS):
+        raise ValueError("need 1 <= budget <= %d, 1 <= width <= %d and budget * width <= %d"
+                         % (N.UCT_MAX_BUDGET, N.UCT_MAX_WIDTH, N.UCT_MAX_PLAYOUTS))
+    return budget, width
+
+
+def _device_mask(env_mask, B, dev):
+    """env_mask (bool [B] or None) as a contiguous uint8 tensor on `dev`"""
+    mask = None if env_mask is None else torch.as_tensor(env_mask).to(dev, torch.bool).to(torch.uint8).contiguous()
+    if mask is not None and mask.numel() != B:
+        raise ValueError("env_mask must have B entries")
+    return mask
+
+
+def _p(t):
+    return None if t is None else t.data_ptr()
+
+
 def uct_search(env, computation_budget=1000, width=1, prune=True, c=UCB_C, seed=1, env_mask=None, root_table=False,
                workspace=None):
     """The search bot for every env of a BatchedEnv* in ONE launch (ddz_uct_search): root b is env b's position (all three
@@ -228,10 +249,7 @@ def uct_search(env, computation_budget=1000, width=1, prune=True, c=UCB_C, seed=
     The search tree lives in a workspace of ddz_uct_workspace_bytes(B, budget) bytes: `workspace` (a device uint8 tensor
     of at least that size, owned by the caller) or, by default, one cached per stream and kept for the next call (free
     the cache with release_workspaces())."""
-    budget, width = int(computation_budget), int(width)
-    if not (1 <= budget <= N.UCT_MAX_BUDGET and 1 <= width <= N.UCT_MAX_WIDTH and budget * width <= N.UCT_MAX_PLAYOUTS):
-        raise ValueError("need 1 <= budget <= %d, 1 <= width <= %d and budget * width <= %d"
-                         % (N.UCT_MAX_BUDGET, N.UCT_MAX_WIDTH, N.UCT_MAX_PLAYOUTS))
+    budget, width = _check_budget(computation_budget, width)
     B, dev = env.B, env.device
     with torch.cuda.device(dev):
         ln = _ln_table(budget * width, dev)
@@ -243,9 +261,7 @@ def uct_search(env, computation_budget=1000, width=1, prune=True, c=UCB_C, seed=
             ws = workspace
             if ws.device != dev or ws.dtype != torch.uint8 or not ws.is_contiguous() or ws.numel() < need:
                 raise ValueError("workspace must be a contiguous uint8 tensor of at least %d bytes on %s" % (need, dev))
-        mask = None if env_mask is None else torch.as_tensor(env_mask).to(dev, torch.bool).to(torch.uint8).contiguous()
-        if mask is not None and mask.numel() != B:
-            raise ValueError("env_mask must have B entries")
+        mask = _device_mask(env_mask, B, dev)
         choice = torch.empty(B, dtype=torch.int32, device=dev)
         moves = torch.empty(B, dtype=torch.int64, device=dev)
         S = min(budget, N.MAX_LEGAL)
@@ -253,9 +269,93 @@ def uct_search(env, computation_budget=1000, width=1, prune=True, c=UCB_C, seed=
         if root_table:
             tab = (torch.zeros(B, dtype=torch.int32, device=dev), torch.zeros((B, S), dtype=torch.int64, device=dev),
                    torch.zeros((B, S), dtype=torch.int32, device=dev), torch.zeros((B, S), dtype=torch.int32, device=dev))
-        p = lambda t: None if t is None else t.data_ptr()
-        N.check(N.lib.ddz_uct_search(p(env._state), p(mask), ws.data_ptr(), budget, width, int(bool(prune)), float(c),
+        N.check(N.lib.ddz_uct_search(_p(env._state), _p(mask), ws.data_ptr(), budget, width, int(bool(prune)), float(c),
                                      ln.data_ptr(), int(seed), env.env0, choice.data_ptr(), moves.data_ptr(),
-                                     *(p(t) for t in (tab or (None,) * 4)), S if root_table else 0, B,
+                                     *(_p(t) for t in (tab or (None,) * 4)), S if root_table else 0, B,
                                      stream.cuda_stream), "ddz_uct_search")
     return (choice, moves) + ((tab,) if root_table else ())
+
+
+# ---------------------------------------------------------------------------------------------------- determinized search
+def _check_determinizations(determinizations, B):
+    D = int(determinizations)
+    if not 1 <= D <= N.PIMC_MAX_DETERMINIZATIONS:
+        raise ValueError("need 1 <= determinizations <= %d" % N.PIMC_MAX_DETERMINIZATIONS)
+    if B * D > 2 ** 31 - 1:
+        raise ValueError("B x determinizations must stay below 2^31")
+    return D
+
+
+def _state_slice(env, b0, n):
+    """a state buffer of its own holding envs b0 .. b0 + n - 1 of env (the state is struct-of-arrays, so a range of envs
+    is not a contiguous part of it); the whole state when the range is the whole batch"""
+    if b0 == 0 and n == env.B:
+        return env._state
+    out = torch.empty(N.lib.ddz_state_bytes(n) // 4, dtype=torch.int32, device=env.device)
+    f, meta = env._fields()
+    out[: 18 * n].view(torch.int64).view(9, n).copy_(f[:, b0:b0 + n])
+    out[18 * n: 19 * n].copy_(meta[b0:b0 + n])
+    return out
+
+
+def determinize(env, determinizations, seed=1, env_mask=None):
+    """ddz_determinize: the raw state (int32 tensor of ddz_state_bytes(B * D) bytes) of B * D full-information envs, env
+    b * D + d being determinization d of env b -- its mover's hand, hist, recent and meta, the two hidden hands replaced by
+    a uniformly random split of the cards the mover has not seen (Philox keyed by (seed, (env.env0 + b) * D + d)).
+    Masked-out and finished envs are copied unchanged; envs no deal agrees with are copied as finished with the sticky error
+    bit and counted in env.stats[7]."""
+    B, dev = env.B, env.device
+    D = _check_determinizations(determinizations, B)
+    with torch.cuda.device(dev):
+        out = torch.empty(N.lib.ddz_state_bytes(B * D) // 4, dtype=torch.int32, device=dev)
+        mask = _device_mask(env_mask, B, dev)
+        N.check(N.lib.ddz_determinize(env._state.data_ptr(), _p(mask), D, int(seed), env.env0, out.data_ptr(),
+                                      env.stats.data_ptr(), B, torch.cuda.current_stream(dev).cuda_stream), "ddz_determinize")
+    return out
+
+
+def pimc_search(env, determinizations=16, computation_budget=1000, width=1, prune=True, c=UCB_C, seed=1, env_mask=None,
+                pooled_table=False, max_workspace_bytes=2 ** 31):
+    """The search bot from the player's own view (determinized UCT, perfect-information Monte Carlo): for every env of a
+    BatchedEnv*, `determinizations` (D) complete deals that agree with what the player to move has seen -- its own hand,
+    the cards every role has played, the last hand-outs and the sizes of the other two hands -- each searched as a
+    full-information game by uct_search's algorithm, and the root statistics added up per move.  The real hidden hands
+    are never read: two envs that show the same view get the same answer.
+    Returns (choice int32 [B], moves int64 [B]) with uct_search's conventions (feed choice to env.step(); -1 / ~0 for an
+    env that is masked out, finished, or whose view no deal agrees with -- the last are counted in env.stats[7]);
+    pooled_table=True adds (pooled_visits, pooled_wins), int32 [B, 512] in the order of env.valid_actions().  The answer is
+    the move with the best pooled wins / visits, the lowest list index on exact ties.
+    Roots are searched in chunks of Bc, Bc x D x (budget + 1) x 160 <= max_workspace_bytes (at least one root per chunk);
+    the results do not depend on the chunking.  The env's state, step counter and lists are left as they are."""
+    budget, width = _check_budget(computation_budget, width)
+    B, dev = env.B, env.device
+    D = _check_determinizations(determinizations, 1)
+    if D * budget * width > 2 ** 31 - 1:
+        raise ValueError("determinizations x budget x width must stay below 2^31 (pooled int32 counts)")
+    Bc = max(1, min(B, int(max_workspace_bytes) // (D * (budget + 1) * N.UCT_NODE_BYTES), (2 ** 31 - 1) // D))
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        ln = _ln_table(budget * width, dev)
+        mask = _device_mask(env_mask, B, dev)
+        ws = _workspace(N.lib.ddz_uct_workspace_bytes(Bc * D, budget), dev, stream)
+        sub = torch.empty(N.lib.ddz_state_bytes(Bc * D) // 4, dtype=torch.int32, device=dev)
+        tree_choice = torch.empty(Bc * D, dtype=torch.int32, device=dev)
+        choice = torch.empty(B, dtype=torch.int32, device=dev)
+        moves = torch.empty(B, dtype=torch.int64, device=dev)
+        tab = None
+        if pooled_table:
+            tab = tuple(torch.empty((B, N.MAX_LEGAL), dtype=torch.int32, device=dev) for _ in range(2))
+        for b0 in range(0, B, Bc):
+            n = min(Bc, B - b0)
+            m = None if mask is None else mask[b0:b0 + n]
+            env0 = (env.env0 + b0) & (2 ** 64 - 1)
+            N.check(N.lib.ddz_determinize(_state_slice(env, b0, n).data_ptr(), _p(m), D, int(seed), env0, sub.data_ptr(),
+                                          env.stats.data_ptr(), n, stream), "ddz_determinize")
+            N.check(N.lib.ddz_uct_search(sub.data_ptr(), _p(None if m is None else m.repeat_interleave(D)), ws.data_ptr(),
+                                         budget, width, int(bool(prune)), float(c), ln.data_ptr(), int(seed),
+                                         (env0 * D) & (2 ** 64 - 1), tree_choice.data_ptr(), None, None, None, None, None,
+                                         0, n * D, stream), "ddz_uct_search")
+            N.check(N.lib.ddz_uct_pool(ws.data_ptr(), budget, D, choice[b0:].data_ptr(), moves[b0:].data_ptr(),
+                                       *(None if t is None else t[b0:].data_ptr() for t in (tab or (None, None))), n,
+                                       stream), "ddz_uct_pool")
+    return (choice, moves) + ((tab,) if pooled_table else ())

@@ -42,7 +42,8 @@
 extern "C" {
 #endif
 
-#define DDZ_ABI_VERSION 3   /* 3: ddz_mcts_moves, ddz_playout_pruned, ddz_q_features (+ ddz_uct_search, ddz_uct_workspace_bytes:
+#define DDZ_ABI_VERSION 3   /* 3: ddz_mcts_moves, ddz_playout_pruned, ddz_q_features (+ ddz_uct_search, ddz_uct_workspace_bytes,
+                            * ddz_determinize, ddz_uct_pool:
                             * new entry points only, backward compatible).  2: ddz_mpipe_*, ddz_set_tile_order, ddz_prob_form; cut lists are played
                             * from their visible part */
 #define DDZ_MAX_LEGAL 512  /* upper bound of legal moves of one decision (worst known hand: 497) */
@@ -238,6 +239,43 @@ int ddz_uct_search(const void* state, const uint8_t* env_mask, void* workspace, 
                    const double* ln_table, uint64_t seed, uint64_t env0, int32_t* choice, uint64_t* move,
                    int32_t* root_n, uint64_t* root_moves, int32_t* root_visits, int32_t* root_wins, int root_stride,
                    int B, void* stream);
+
+/* Search from the player's own view (determinized UCT, perfect-information Monte Carlo): sample D complete deals that agree
+ * with what the player to move has seen, search each with ddz_uct_search, add up the root statistics per move.
+ *
+ * ddz_determinize: out_state holds ddz_state_bytes(B * D) bytes; env b * D + d is determinization d of env b.  The mover's
+ * hand (role m = meta bits 0-1), hist[3], recent[3] and meta are copied from env b; the hands of roles a = (m+1)%3 and
+ * c = (m+2)%3 become a random split of the UNSEEN cards = full deck - hand[m] - hist[0] - hist[1] - hist[2], a getting as
+ * many cards as its hand holds and c the rest.  Draw rule: the unseen cards are walked in rank order 0..14, one physical
+ * card at a time, j = 0 .. U-1; card j goes to a when
+ *     philox(seed, (env0 + b) * D + d, 0xC0000000 + j) % (ra + rc) < ra
+ * (ra, rc: the slots still open in each hand), else to c; a draw is taken for every card, also when one side is full.
+ * This is selection sampling: every split of the (distinguishable) unseen cards into those two sizes is equally likely, up
+ * to the modulo bias of a 32-bit draw.  The Philox stream (seed, (env0 + b) * D + d) is the one ddz_uct_search uses for
+ * that determinization when it is called with env0' = (env0 + b0) * D over the B * D envs; the ranges cannot collide:
+ * determinization draws take steps 0xC0000000 .. +36, tree draws start at 0x80000000 and a tree takes fewer than 2^30 of
+ * them, playouts take steps below 400.
+ * Masked-out (env_mask uint8[B], NULL = all) and finished envs are copied unchanged and take no draw.  A root whose view no
+ * deal agrees with (a negative unseen count for a rank, or U != |hand[a]| + |hand[c]|, e.g. a full-information env with
+ * zero hist) is copied with meta bits 2 (done) and 5 (sticky error) set in all D copies, and stats[7] (stats may be NULL)
+ * counts it once; the search then skips those copies as finished.
+ * NULL state / out_state, B <= 0, D outside 1..DDZ_PIMC_MAX_DETERMINIZATIONS or B * D > INT_MAX: DDZ_E_ARG before any CUDA
+ * call.
+ *
+ * ddz_uct_pool: `workspace` as written by ddz_uct_search over B * D roots (tree b * D + d, same budget).  For root b, the
+ * root children (parent 0) of every tree with nnodes > 0 add their visits and wins under their canonical `index`
+ * (duplicate pruned entries of one tree add up too): pooled_visits / pooled_wins int32 [B][DDZ_MAX_LEGAL] (optional, each
+ * may be NULL), in the order of the env's canonical legal list.  choice[b] = the index with the best pooled wins / visits
+ * among those with visits > 0 (W_i * V_j against W_j * V_i in 64 bits; exact ties go to the LOWEST index), -1 when no tree
+ * of b was searched; move[b] (optional) = the packed move at that index (select_legal over the root's hand and trick), or
+ * ~0.  NULL workspace / choice, B <= 0, budget outside 1..DDZ_UCT_MAX_BUDGET, D outside 1..DDZ_PIMC_MAX_DETERMINIZATIONS,
+ * B * D > INT_MAX or D * budget > INT_MAX: DDZ_E_ARG before any CUDA call.  The int32 sums cannot overflow when
+ * D * budget * width <= 2^31 - 1. */
+#define DDZ_PIMC_MAX_DETERMINIZATIONS 4096
+int ddz_determinize(const void* state, const uint8_t* env_mask, int D, uint64_t seed, uint64_t env0, void* out_state,
+                    int64_t* stats, int B, void* stream);
+int ddz_uct_pool(const void* workspace, int budget, int D, int32_t* choice, uint64_t* move, int32_t* pooled_visits,
+                 int32_t* pooled_wins, int B, void* stream);
 
 /* Env.batch_arr2onehot over packed moves (envi.py:113,140-146): out float32[n][15][4] */
 int ddz_encode_actions(const uint64_t* actions_u64, int64_t n, float* out, void* stream);
