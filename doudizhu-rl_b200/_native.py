@@ -27,7 +27,7 @@ EXPORTS = ("ddz_abi_version", "ddz_prob_form", "ddz_set_tile_order", "ddz_face_c
            "ddz_pipe_step", "ddz_pipe_wait", "ddz_pipe_refill", "ddz_pipe_flush", "ddz_rollout_steps", "ddz_encode_state_actions", "ddz_legal_count", "ddz_legal_emit", "ddz_rows_alloc", "ddz_rows_free",
            "ddz_mpipe_create", "ddz_mpipe_destroy", "ddz_mpipe_step", "ddz_mpipe_wait", "ddz_mpipe_refill", "ddz_mpipe_flush", "ddz_mpipe_join",
            "ddz_mcts_moves", "ddz_playout_pruned", "ddz_q_features", "ddz_uct_workspace_bytes", "ddz_uct_search",
-           "ddz_determinize", "ddz_uct_pool")
+           "ddz_determinize", "ddz_uct_pool", "ddz_encode_face_gather")
 
 lib = C.CDLL(LIB_PATH)
 _missing = [name for name in EXPORTS if not hasattr(lib, name)]
@@ -67,6 +67,9 @@ lib.ddz_rollout_steps.argtypes = [_vp, _vp, _i, _i, _vp, _vp, _vp, _i, _u64, _u6
 lib.ddz_legal_moves.argtypes = [_vp, _vp, _vp, _vp, _vp, _i64, _vp, _i, _vp]
 lib.ddz_encode_actions.argtypes = [_vp, _i64, _vp, _vp]
 lib.ddz_encode_face.argtypes = [_vp, _i, _vp, _i, _vp]
+lib.ddz_encode_face_gather.argtypes = [_vp, _i, _vp, _i64, _vp, _vp, _vp, _i, _i, _vp]
+ROWS_SPLIT, ROWS_CONCAT = 0, 1
+STATE_WORDS = 19                     # int32 words of one env in a library state (uint64 hand/hist/recent [3], uint32 meta)
 lib.ddz_kth_moves.argtypes = [_vp, _vp, _vp, _vp, _vp, _i, _vp]
 lib.ddz_playout.argtypes = [_vp, _i, _u64, _u64, _u32, _vp, _vp, _vp, _i, _vp]
 lib.ddz_playout_pruned.argtypes = lib.ddz_playout.argtypes

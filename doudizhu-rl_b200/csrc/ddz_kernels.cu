@@ -905,13 +905,67 @@ __global__ void __launch_bounds__(kQThreads) k_q_features(const void* state, con
     }
 }
 
+// the thermometer one-hot of rank `rank` of a packed move (envi.py:140-146, batch_arr2onehot)
+DDZ_DEV float4 move_thermo(uint64_t move, int rank) {
+    const uint32_t c = (uint32_t)(move >> (4 * rank)) & 15u;
+    return make_float4(c > 0 ? 1.f : 0.f, c > 1 ? 1.f : 0.f, c > 2 ? 1.f : 0.f, c > 3 ? 1.f : 0.f);
+}
+
 __global__ void __launch_bounds__(256) k_encode_actions(const uint64_t* __restrict__ actions, long long n,
                                                         float4* __restrict__ out) {
     long long nvec = n * 15;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += (long long)gridDim.x * blockDim.x) {
         long long row = i / 15; int rank = (int)(i - row * 15);
-        uint32_t c = (uint32_t)(actions[row] >> (4 * rank)) & 15u;
-        out[i] = make_float4(c > 0 ? 1.f : 0.f, c > 1 ? 1.f : 0.f, c > 2 ? 1.f : 0.f, c > 3 ? 1.f : 0.f);
+        out[i] = move_thermo(actions[row], rank);
+    }
+}
+
+// Replay decode (ddz_encode_face_gather): k_face over env rows[i] of a stored state, plus the one-hot row of that env's
+// packed move.  CONCAT: face [n][C+1] rows with the move row last (k_state_actions' rows); else face [n][C] rows and, when
+// move_rows != NULL, move_rows [n].  A row outside [0, B) reads nothing and gives zero rows.
+template <int V, bool CONCAT>
+__global__ void __launch_bounds__(kEnvs) k_face_gather(const void* state, const int64_t* __restrict__ rows, long long n,
+                                                       const uint64_t* __restrict__ moves, float4* __restrict__ face,
+                                                       float4* __restrict__ move_rows, int B) {
+    constexpr int C = FaceCfg<V>::C, R = CONCAT ? C + 1 : C;   // R: rows per sample in `face`
+    __shared__ uint64_t s_planes[kEnvs * (C + 1)];              // the C face planes, then the move
+    __shared__ float s_p[kEnvs * 2];
+    const int tid = threadIdx.x;
+    const long long i0 = (long long)blockIdx.x * kEnvs;
+    if (i0 + tid < n) {
+        const long long b = rows[i0 + tid];
+        uint64_t pl[C], mv = 0; float p[2] = {0.f, 0.f};
+        if (b >= 0 && b < B) {
+            const Env e = load_env(view_of(const_cast<void*>(state), B), (int)b);
+            face_planes<V>(e, pl, p);
+            if (moves) mv = moves[b];
+        } else {
+#pragma unroll
+            for (int c = 0; c < C; c++) pl[c] = 0;
+        }
+#pragma unroll
+        for (int c = 0; c < C; c++) s_planes[tid * (C + 1) + c] = pl[c];
+        s_planes[tid * (C + 1) + C] = mv;
+        s_p[tid * 2] = p[0]; s_p[tid * 2 + 1] = p[1];
+    }
+    __syncthreads();
+    const int ns = (int)min((long long)kEnvs, n - i0);
+    float4* dst = face + (size_t)i0 * R * 15;
+    const int nvec = ns * R * 15;
+    for (int i = tid; i < nvec; i += kEnvs) {
+        const int row = i / 15, rank = i - row * 15;
+        const int smp = row / R, c = row - smp * R;
+        if (CONCAT && c == C) { dst[i] = move_thermo(s_planes[smp * (C + 1) + C], rank); continue; }
+        const float s = (c >= C - 2) ? s_p[smp * 2 + (c - (C - 2))] : 1.f;
+        const float4 q = lut_entry((int)((uint32_t)(s_planes[smp * (C + 1) + c] >> (4 * rank)) & 15u));
+        dst[i] = make_float4(q.x * s, q.y * s, q.z * s, q.w * s);
+    }
+    if (!CONCAT && move_rows) {
+        float4* mdst = move_rows + (size_t)i0 * 15;
+        for (int i = tid; i < ns * 15; i += kEnvs) {
+            const int smp = i / 15, rank = i - smp * 15;
+            mdst[i] = move_thermo(s_planes[smp * (C + 1) + C], rank);
+        }
     }
 }
 
@@ -1581,6 +1635,18 @@ const DriverApi& driver_api() {
 }
 }  // namespace
 
+template <int V>
+static int launch_face_gather(const void* state, const int64_t* rows, int64_t n, const uint64_t* moves, float* face,
+                              float* move_rows, int layout, int B, cudaStream_t st) {
+    const unsigned grid = (unsigned)((n + kEnvs - 1) / kEnvs);
+    if (layout == DDZ_ROWS_CONCAT)
+        k_face_gather<V, true><<<grid, kEnvs, 0, st>>>(state, rows, n, moves, (float4*)face, nullptr, B);
+    else
+        k_face_gather<V, false><<<grid, kEnvs, 0, st>>>(state, rows, n, moves, (float4*)face, (float4*)move_rows, B);
+    DDZ_LAUNCH_CHECK("k_face_gather");
+    return 0;
+}
+
 extern "C" {
 
 #ifdef DDZ_TRACE
@@ -2186,6 +2252,24 @@ int ddz_encode_face(const void* state, int variant, float* face, int B, void* st
     }
     DDZ_LAUNCH_CHECK("k_face");
     return 0;
+}
+
+int ddz_encode_face_gather(const void* state, int variant, const int64_t* rows, int64_t n, const uint64_t* moves,
+                           float* face, float* move_rows, int layout, int B, void* stream) {
+    if (n < 0 || B <= 0 || ddz_face_channels(variant) < 0) return DDZ_E_ARG;
+    if (layout != DDZ_ROWS_SPLIT && layout != DDZ_ROWS_CONCAT) return DDZ_E_ARG;
+    if (n > 0 && (!state || !rows || !face)) return DDZ_E_ARG;
+    if (layout == DDZ_ROWS_CONCAT && (!moves || move_rows)) return DDZ_E_ARG;
+    if (layout == DDZ_ROWS_SPLIT && move_rows && !moves) return DDZ_E_ARG;
+    if ((n + kEnvs - 1) / kEnvs > INT_MAX) return DDZ_E_ARG;
+    if (n == 0) return 0;
+    const cudaStream_t st = (cudaStream_t)stream;
+    switch (variant) {
+        case 0: return launch_face_gather<0>(state, rows, n, moves, face, move_rows, layout, B, st);
+        case 1: return launch_face_gather<1>(state, rows, n, moves, face, move_rows, layout, B, st);
+        case 2: return launch_face_gather<2>(state, rows, n, moves, face, move_rows, layout, B, st);
+        default: return launch_face_gather<3>(state, rows, n, moves, face, move_rows, layout, B, st);
+    }
 }
 
 }  // extern "C"

@@ -20,8 +20,8 @@ import time
 import torch
 
 from .agent import BatchedGreedyPolicy
-from .env import random_deals
-from .trainer import ReplayBuffer, TransitionCollector, td_step
+from .env import VARIANT_CHANNELS, random_deals
+from .trainer import PackedReplayBuffer, ReplayBuffer, TransitionCollector, td_step
 
 # config.py:7-14
 GAMMA = 0.95
@@ -41,9 +41,12 @@ class BatchedDQN:
     and verbs (`perceive`, `e_greedy_action`, `greedy_action`, `update_epsilon`, `update_target`)."""
 
     def __init__(self, net_cls, face_channels, device, replay_size=REPLAY_SIZE, batch_size=BATCH_SIZE, gamma=GAMMA,
-                 lr=1e-4, decay=DECAY, update_target_every=UPDATE_TARGET_EVERY, seed=0, fused=False, precision="fp32"):
+                 lr=1e-4, decay=DECAY, update_target_every=UPDATE_TARGET_EVERY, seed=0, fused=False, precision="fp32",
+                 replay="float"):
         """fused=True: the moves are scored by agent.FusedQScorer (ddz_q_features + two GEMMs, for the NetComplicated family of
-        net.py) instead of the module's forward; its tables are rebuilt from the weights after every update."""
+        net.py) instead of the module's forward; its tables are rebuilt from the weights after every update.
+        replay="packed": the replay buffer is a trainer.PackedReplayBuffer (transitions as packed states and moves, 176 B
+        each; perceive takes what TransitionCollector(packed=True) emits); "float" (default): trainer.ReplayBuffer."""
         self.device = torch.device(device)
         self.epsilon = EPSILON_HIGH
         self.batch_size, self.gamma, self.decay, self.update_target_every = int(batch_size), float(gamma), decay, update_target_every
@@ -51,7 +54,12 @@ class BatchedDQN:
         self.target_net = net_cls().to(self.device)
         self.target_net.load_state_dict(self.policy_net.state_dict())
         self.optimizer = torch.optim.Adam(self.policy_net.parameters(), lr)
-        self.replay_buffer = ReplayBuffer(replay_size, face_channels, self.device)
+        if replay == "packed":
+            self.replay_buffer = PackedReplayBuffer(replay_size, VARIANT_CHANNELS.index(face_channels), self.device)
+        elif replay == "float":
+            self.replay_buffer = ReplayBuffer(replay_size, face_channels, self.device)
+        else:
+            raise ValueError("replay must be 'float' or 'packed', not %r" % (replay,))
         self._policy = BatchedGreedyPolicy(self.policy_net, epsilon=0.0, seed=seed, fused=fused, precision=precision)
         self._gen = torch.Generator(device=self.device)
         self._gen.manual_seed(int(seed) + 1)
@@ -98,16 +106,23 @@ class BatchedGame:
     search_dict (optional) seats the search bot: role -> keyword arguments of search.pimc_search, e.g.
     {"lord": {"determinizations": 8, "computation_budget": 125}}; that role plays from its own view (determinized UCT),
     or with "determinizations": 0 the full-information search.uct_search, which sees every hand.  A role has a net or a
-    search entry, not both."""
+    search entry, not both.
+    replay="packed" keeps the learning roles' transitions as packed states and moves (trainer.PackedReplayBuffer, 176 B a
+    transition instead of 2 * 240 * (C + 1) + 8 B): `dqns_dict[role]` is then called with the extra keyword replay="packed".
+    Set the capacity through the DQN class, e.g. functools.partial(BatchedDQN, replay_size=10_000_000)."""
 
     def __init__(self, env_cls, nets_dict, dqns_dict, reward_dict=None, train_dict=None, preload=None, seed=None,
-                 debug=False, num_envs=4096, pool_games=8, deals=None, device=None, updates_per_step=1, search_dict=None):
+                 debug=False, num_envs=4096, pool_games=8, deals=None, device=None, updates_per_step=1, search_dict=None,
+                 replay="float"):
         if reward_dict is None:
             reward_dict = {"lord": 100, "down": 50, "up": 50}
         if train_dict is None:
             train_dict = {"lord": True, "down": True, "up": True}
         preload = preload or {}
         assert not (nets_dict.keys() ^ dqns_dict.keys()), "Net and DQN must match"
+        if replay not in ("float", "packed"):
+            raise ValueError("replay must be 'float' or 'packed', not %r" % (replay,))
+        self.packed = replay == "packed"
         self.search_dict = {r: dict(kw) for r, kw in (search_dict or {}).items()}
         for role in self.search_dict:
             if role not in ROLE_INDEX:
@@ -124,7 +139,8 @@ class BatchedGame:
         self._collectors = {}
         for role in ("lord", "down", "up"):
             if nets_dict.get(role):
-                agent = dqns_dict[role](nets_dict[role], self.env.C, self.device)
+                extra = {"replay": "packed"} if self.packed else {}      # custom DQN classes keep their signature
+                agent = dqns_dict[role](nets_dict[role], self.env.C, self.device, **extra)
                 setattr(self, role, agent)
                 setattr(self, "%s_train" % role, bool(train_dict.get(role)))
                 if preload.get(role):
@@ -132,7 +148,8 @@ class BatchedGame:
                         net.load(preload[role])
                 if train_dict.get(role):
                     self._collectors[role] = TransitionCollector(self.env, role=ROLE_INDEX[role],
-                                                                 reward=float(reward_dict[role]))
+                                                                 reward=float(reward_dict[role]),
+                                                                 **({"packed": True} if self.packed else {}))
         # counters with the reference's names (game.py:20-26)
         self.lord_wins, self.down_wins, self.up_wins = [], [], []
         self.up_total_wins = self.lord_total_wins = self.down_total_wins = 0
@@ -202,9 +219,14 @@ class BatchedGame:
             choice = torch.where(mine, k.clamp(min=0), choice)
             if training:
                 kg = agent.greedy_action(env, q).to(torch.int64).clamp(min=0)
-                keep = (cnt > 0)[:, None, None]
-                a0 = acts[(off[:-1] + k.clamp(min=0)).clamp(max=last)] * keep
-                a1 = acts[(off[:-1] + kg).clamp(max=last)] * keep
+                if self.packed:                      # packed moves, 0 (a pass row of zeros) where there is no move
+                    au, keep = env.actions_packed, cnt > 0
+                    a0 = au[(off[:-1] + k.clamp(min=0)).clamp(max=last)] * keep
+                    a1 = au[(off[:-1] + kg).clamp(max=last)] * keep
+                else:
+                    keep = (cnt > 0)[:, None, None]
+                    a0 = acts[(off[:-1] + k.clamp(min=0)).clamp(max=last)] * keep
+                    a1 = acts[(off[:-1] + kg).clamp(max=last)] * keep
                 pending.append((role, self._collectors[role].on_turn(a0, a1)))
         for role, kw in self.search_dict.items():
             mine = (seat == ROLE_INDEX[role]) & live

@@ -43,7 +43,7 @@ extern "C" {
 #endif
 
 #define DDZ_ABI_VERSION 3   /* 3: ddz_mcts_moves, ddz_playout_pruned, ddz_q_features (+ ddz_uct_search, ddz_uct_workspace_bytes,
-                            * ddz_determinize, ddz_uct_pool:
+                            * ddz_determinize, ddz_uct_pool, ddz_encode_face_gather:
                             * new entry points only, backward compatible).  2: ddz_mpipe_*, ddz_set_tile_order, ddz_prob_form; cut lists are played
                             * from their visible part */
 #define DDZ_MAX_LEGAL 512  /* upper bound of legal moves of one decision (worst known hand: 497) */
@@ -375,6 +375,24 @@ int ddz_rows_free(void* ptr, size_t mapped_bytes);
 
 /* env.face only (envi.py:87-217) */
 int ddz_encode_face(const void* state, int variant, float* face, int B, void* stream);
+
+/* Replay decode: the float transition rows a DQN minibatch needs (dqn.py:22-29 sample), rebuilt from packed states and moves.
+ * A replay buffer that keeps each transition as two packed states (2 x 76 B) and two packed moves instead of float faces
+ * and one-hot rows (2 x 240 (C + 1) B) decodes only the sampled rows, in one launch.
+ * Sample i takes env rows[i] of `state` (a state of B envs) and its move moves[rows[i]] (uint64 [B]); rows are arbitrary,
+ * duplicates and any order included.
+ *   DDZ_ROWS_SPLIT:  face float32 [n][C][15][4] = what ddz_encode_face writes for that env, bit for bit; move_rows (optional)
+ *                    float32 [n][15][4] = what ddz_encode_actions writes for that move (a pass, 0, is the zero row:
+ *                    the reference's a1 = zeros of a terminal transition, game.py:123-124);
+ *   DDZ_ROWS_CONCAT: face float32 [n][C+1][15][4], rows [face | move one-hot] = the Q-network input of net.py:88-90, the
+ *                    rows ddz_encode_state_actions writes (move_rows must be NULL).
+ * A row outside [0, B) gives all-zero rows and reads nothing.  n = 0 returns 0 without a launch.  NULL state / rows / face
+ * with n > 0, n < 0, B <= 0, an unknown variant or layout, moves == NULL with DDZ_ROWS_CONCAT or with move_rows != NULL,
+ * move_rows != NULL with DDZ_ROWS_CONCAT: DDZ_E_ARG before any CUDA call.  Form-B builds write the form-B rows. */
+#define DDZ_ROWS_SPLIT 0
+#define DDZ_ROWS_CONCAT 1
+int ddz_encode_face_gather(const void* state, int variant, const int64_t* rows, int64_t n, const uint64_t* moves,
+                           float* face, float* move_rows, int layout, int B, void* stream);
 
 #ifdef __cplusplus
 }
