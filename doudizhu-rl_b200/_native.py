@@ -27,7 +27,7 @@ EXPORTS = ("ddz_abi_version", "ddz_prob_form", "ddz_set_tile_order", "ddz_face_c
            "ddz_pipe_step", "ddz_pipe_wait", "ddz_pipe_refill", "ddz_pipe_flush", "ddz_rollout_steps", "ddz_encode_state_actions", "ddz_legal_count", "ddz_legal_emit", "ddz_rows_alloc", "ddz_rows_free",
            "ddz_mpipe_create", "ddz_mpipe_destroy", "ddz_mpipe_step", "ddz_mpipe_wait", "ddz_mpipe_refill", "ddz_mpipe_flush", "ddz_mpipe_join",
            "ddz_mcts_moves", "ddz_playout_pruned", "ddz_q_features", "ddz_uct_workspace_bytes", "ddz_uct_search",
-           "ddz_determinize", "ddz_uct_pool", "ddz_encode_face_gather")
+           "ddz_determinize", "ddz_uct_pool", "ddz_encode_face_gather", "ddz_move_ids", "ddz_moves_of_ids", "ddz_legal_mask")
 
 lib = C.CDLL(LIB_PATH)
 _missing = [name for name in EXPORTS if not hasattr(lib, name)]
@@ -117,6 +117,11 @@ lib.ddz_mpipe_refill.argtypes = [_vp, C.POINTER(GroupStep), C.POINTER(_vp), C.PO
 lib.ddz_mpipe_flush.argtypes = [_vp, C.POINTER(GroupStep)]
 lib.ddz_mpipe_join.argtypes = [_vp, _vp]
 lib.ddz_select_actions.argtypes = [_vp, _vp, C.c_float, _u64, _u64, _u32, _vp, _i, _vp]
+lib.ddz_move_ids.argtypes = [_vp, _i64, _vp, _vp]
+lib.ddz_moves_of_ids.argtypes = [_vp, _i64, _vp, _vp]
+lib.ddz_legal_mask.argtypes = [_vp, _vp, _i64, _i, _vp, _vp, _i, _vp]
+NUM_ACTION_IDS, MOVE_INVALID, MASK_WORDS = 13551, 0xFFFFFFFFFFFFFFFF, 424
+MASK_BITS, MASK_BYTES = 0, 1
 
 if lib.ddz_abi_version() != ABI_VERSION:
     raise ImportError("libddz_b200.so ABI %d != binding %d: rebuild" % (lib.ddz_abi_version(), ABI_VERSION))

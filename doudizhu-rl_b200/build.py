@@ -5,7 +5,8 @@ import subprocess
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-SRC = [os.path.join(HERE, "csrc", f) for f in ("ddz_kernels.cu", "ddz_device.cuh", "ddz_flat.cuh")] + \
+SRC = [os.path.join(HERE, "csrc", f) for f in ("ddz_kernels.cu", "ddz_device.cuh", "ddz_flat.cuh", "ddz_ids.cuh",
+                                                "ddz_action_ids.inc")] + \
       [os.path.join(ROOT, "include", "ddz_b200.h")]
 LIB = os.path.join(HERE, "libddz_b200.so")
 LIB_FORM_B = os.path.join(HERE, "libddz_b200_formB.so")   # the other layout of the probability planes (-DDDZ_PROB_FORM_B)

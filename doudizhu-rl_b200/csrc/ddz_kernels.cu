@@ -39,6 +39,7 @@
 #include <math_constants.h>
 #include "ddz_flat.cuh"
 #include "ddz_search.cuh"
+#include "ddz_ids.cuh"
 
 namespace ddz {
 
@@ -1521,6 +1522,63 @@ __global__ void __launch_bounds__(256) k_select_actions(const float* __restrict_
     choice[b] = best;
 }
 
+// Action ids (ddz_ids.cuh), one thread per element.
+__global__ void __launch_bounds__(256) k_move_ids(const uint64_t* __restrict__ moves, long long n, int32_t* __restrict__ ids) {
+    for (long long i = blockIdx.x * 256ll + threadIdx.x; i < n; i += (long long)gridDim.x * 256) ids[i] = move_id(moves[i]);
+}
+__global__ void __launch_bounds__(256) k_moves_of_ids(const int32_t* __restrict__ ids, long long n, uint64_t* __restrict__ moves) {
+    for (long long i = blockIdx.x * 256ll + threadIdx.x; i < n; i += (long long)gridDim.x * 256) moves[i] = move_of_id(ids[i]);
+}
+
+// Legal-id mask rows, one warp per env.  The warp turns the env's stored list into ids in shared memory (they strictly
+// increase), then every lane writes 16-byte pieces lane, lane + 32, ... of the row (coalesced), finding the ids of each piece
+// by a merge walk that only moves forward.  Every byte of the row is stored once: no zero-fill pass, no atomics.
+constexpr int kMaskWarps = 8;
+DDZ_DEV bool has_id(const int16_t* ids, int n, int id) {
+    int lo = 0, hi = n;                                    // first entry >= id
+    while (lo < hi) { const int mid = (lo + hi) >> 1; if (ids[mid] < id) lo = mid + 1; else hi = mid; }
+    return lo < n && ids[lo] == id;
+}
+template <bool BYTES>
+__global__ void __launch_bounds__(kMaskWarps * 32) k_legal_mask(const int32_t* __restrict__ offsets,
+                                                                const uint64_t* __restrict__ actions, long long cap,
+                                                                void* out, int64_t* stats, int B) {
+    __shared__ int16_t sids[kMaskWarps][DDZ_MAX_LEGAL];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int b = blockIdx.x * kMaskWarps + w;
+    if (b >= B) return;
+    int16_t* ids = sids[w];
+    const long long lo = offsets[b], full = max(0ll, (long long)offsets[b + 1] - lo);
+    const long long stored = max(0ll, min(full, cap - lo));
+    if (lane == 0 && stored < full && stats) atomicAdd((unsigned long long*)&stats[7], 1ull);
+    const int n = (int)min(stored, (long long)DDZ_MAX_LEGAL);
+    for (int i = lane; i < n; i += 32) ids[i] = (int16_t)move_id(actions[lo + i]);
+    __syncwarp();
+    constexpr int kSpan = BYTES ? 16 : 128;                // ids per 16-byte piece
+    int p = 0;
+    auto piece = [&](int base) {                           // the 16 bytes of ids [base, base + kSpan)
+        uint32_t v[4] = {0u, 0u, 0u, 0u};
+        while (p < n && ids[p] < base) p++;
+        for (; p < n && ids[p] < base + kSpan; p++) {
+            const int d = ids[p] - base;                   // < 0 only for an entry that is not a move (-1)
+            if (d >= 0) { if (BYTES) v[d >> 2] |= 1u << (8 * (d & 3)); else v[d >> 5] |= 1u << (d & 31); }
+        }
+        return make_uint4(v[0], v[1], v[2], v[3]);
+    };
+    if (!BYTES) {
+        uint4* row = reinterpret_cast<uint4*>(out) + (size_t)b * (DDZ_MASK_WORDS / 4);
+        for (int c = lane; c < DDZ_MASK_WORDS / 4; c += 32) row[c] = piece(c * kSpan);
+    } else {
+        uint8_t* row = reinterpret_cast<uint8_t*>(out) + (size_t)b * DDZ_NUM_ACTION_IDS;
+        const int head = (int)((0u - (uint32_t)reinterpret_cast<uintptr_t>(row)) & 15u);   // bytes before a 16-byte boundary
+        const int nmid = (DDZ_NUM_ACTION_IDS - head) >> 4, tail = head + 16 * nmid;
+        if (lane < head) row[lane] = has_id(ids, n, lane);
+        if (lane >= 16 && tail + lane - 16 < DDZ_NUM_ACTION_IDS) row[tail + lane - 16] = has_id(ids, n, tail + lane - 16);
+        uint4* mid = reinterpret_cast<uint4*>(row + head);
+        for (int c = lane; c < nmid; c += 32) mid[c] = piece(head + c * kSpan);
+    }
+}
+
 }  // namespace ddz
 
 // ------------------------------------------------------------------------------------------------
@@ -2270,6 +2328,37 @@ int ddz_encode_face_gather(const void* state, int variant, const int64_t* rows, 
         case 2: return launch_face_gather<2>(state, rows, n, moves, face, move_rows, layout, B, st);
         default: return launch_face_gather<3>(state, rows, n, moves, face, move_rows, layout, B, st);
     }
+}
+
+static unsigned elementwise_grid(int64_t n) { const int64_t g = (n + 255) / 256; return (unsigned)(g < 148 * 16 ? g : 148 * 16); }
+
+int ddz_move_ids(const uint64_t* moves, int64_t n, int32_t* ids, void* stream) {
+    if (n < 0 || (n > 0 && (!moves || !ids))) return DDZ_E_ARG;
+    if (n == 0) return 0;
+    k_move_ids<<<elementwise_grid(n), 256, 0, (cudaStream_t)stream>>>(moves, n, ids);
+    DDZ_LAUNCH_CHECK("k_move_ids");
+    return 0;
+}
+
+int ddz_moves_of_ids(const int32_t* ids, int64_t n, uint64_t* moves, void* stream) {
+    if (n < 0 || (n > 0 && (!ids || !moves))) return DDZ_E_ARG;
+    if (n == 0) return 0;
+    k_moves_of_ids<<<elementwise_grid(n), 256, 0, (cudaStream_t)stream>>>(ids, n, moves);
+    DDZ_LAUNCH_CHECK("k_moves_of_ids");
+    return 0;
+}
+
+int ddz_legal_mask(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, int layout, void* out, int64_t* stats,
+                   int B, void* stream) {
+    if (!offsets || !out || B <= 0 || cap < 0 || (cap > 0 && !actions_u64)) return DDZ_E_ARG;
+    if (layout != DDZ_MASK_BITS && layout != DDZ_MASK_BYTES) return DDZ_E_ARG;
+    if (layout == DDZ_MASK_BITS && (reinterpret_cast<uintptr_t>(out) & 15u) != 0) return DDZ_E_ARG;   // 16-byte row stores
+    const unsigned grid = (unsigned)((B + kMaskWarps - 1) / kMaskWarps);
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (layout == DDZ_MASK_BITS) k_legal_mask<false><<<grid, kMaskWarps * 32, 0, st>>>(offsets, actions_u64, cap, out, stats, B);
+    else k_legal_mask<true><<<grid, kMaskWarps * 32, 0, st>>>(offsets, actions_u64, cap, out, stats, B);
+    DDZ_LAUNCH_CHECK("k_legal_mask");
+    return 0;
 }
 
 }  // extern "C"

@@ -9,6 +9,8 @@ reference's game.py / dqn.py / net.py loop runs on them unchanged.
 All arithmetic happens in hand-written sm_100a kernels behind the C-ABI of include/ddz_b200.h; PyTorch only
 owns the buffers and the stream.  There is no CPU fallback.
 """
+from collections import namedtuple
+
 import numpy as np
 import torch
 
@@ -323,6 +325,32 @@ class BatchedEnv:
     def step(self, choice):
         """apply legal move number choice[b] of every env (the index stream of the parity contract)."""
         return self._step(self._to_dev(choice, torch.int32), N.CHOICE_INDEX)
+
+    def legal_ids(self):
+        """int32 [sumN]: the action id (move_ids) of every legal move, in CSR order parallel to valid_actions() -- the ids
+        of one env's list strictly increase."""
+        return move_ids(self.actions_packed, self.device)
+
+    def legal_mask(self, layout="bool"):
+        """One row per env over the 13 551 action ids (ddz_legal_mask; the counterpart of the reference's
+        get_mask_onehot60): "bool" -> bool [B, 13551]; "bits" -> int32 [B, 424], bit id & 31 of word id >> 5.  A finished
+        env has an all-zero row.  The lists are complete (the buffers grow as num_actions does)."""
+        lay = {"bool": N.MASK_BYTES, "bits": N.MASK_BITS}.get(layout)
+        if lay is None:
+            raise ValueError("layout must be 'bool' or 'bits', not %r" % (layout,))
+        self.num_actions
+        shape, dtype = ((self.B, N.NUM_ACTION_IDS), torch.bool) if lay == N.MASK_BYTES else ((self.B, N.MASK_WORDS), torch.int32)
+        out = torch.empty(shape, dtype=dtype, device=self.device)
+        with torch.cuda.device(self.device):
+            N.check(N.lib.ddz_legal_mask(self._p(self._offsets[self._cur]), self._p(self._actions_u64[self._cur]), self.cap,
+                                         lay, out.data_ptr(), self._p(self.stats), self.B, self._stream()), "ddz_legal_mask")
+        return out
+
+    def step_ids(self, ids):
+        """apply the move with action id ids[b] in every env (moves_of_ids, then the DDZ_CHOICE_MOVE step).  An id that is
+        not legal in its env, or outside [0, 13551), is an illegal choice: the env is left as it is, its sticky error bit
+        is set, stats[7] counts it, and debug=True raises."""
+        return self._step(moves_of_ids(self._to_dev(ids, torch.int32), self.device), N.CHOICE_MOVE)
 
     def step_manual(self, onehot_cards):
         """envi.py:63-70: onehot float/int [B,15,4] (a row of valid_actions per env) -> (r, done, cat)."""
@@ -1044,6 +1072,64 @@ def get_moves(hands, lasts, device=None):
         N.check(N.lib.ddz_legal_moves(h.data_ptr(), l.data_ptr(), ws.data_ptr(), offsets.data_ptr(), out.data_ptr(),
                                       cap, None, n, torch.cuda.current_stream(dev).cuda_stream), "ddz_legal_moves")
     return out[: int(offsets[n].item())], offsets
+
+
+# ---------------------------------------------------------------------- action ids (a fixed index per move)
+ActionSpace = namedtuple("ActionSpace", "moves card_py_index id_of_card_py")
+
+
+def _id_device(device):
+    if not torch.cuda.is_available():
+        raise N.DdzError("action ids are computed on a CUDA device")
+    return torch.device(device if device is not None else "cuda:%d" % torch.cuda.current_device())
+
+
+def _as_int_tensor(x, dtype, dev):
+    if isinstance(x, np.ndarray) and x.dtype == np.uint64:
+        x = x.view(np.int64)
+    t = torch.as_tensor(x)
+    if t.dtype == torch.uint64:
+        t = t.view(torch.int64)
+    return t.to(device=dev, dtype=dtype).contiguous()
+
+
+def move_ids(packed, device=None):
+    """Action id of every packed move (include/ddz_b200.h, ddz_move_ids): its index in the universe of 13 551 moves -- the
+    reference's action space (card.py) plus the 24 rocket-kicker moves of r.get_moves, id 0 = pass --, or -1 for a value
+    that is not a move.  packed int64 / uint64 [...] -> int32 [...] on the device."""
+    dev = _id_device(device)
+    p = _as_int_tensor(packed, torch.int64, dev)
+    out = torch.empty(p.shape, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        N.check(N.lib.ddz_move_ids(p.data_ptr(), p.numel(), out.data_ptr(), torch.cuda.current_stream(dev).cuda_stream),
+                "ddz_move_ids")
+    return out
+
+
+def moves_of_ids(ids, device=None):
+    """The packed move of every action id (ddz_moves_of_ids): int [...] -> int64 [...] on the device; an id outside
+    [0, 13551) gives MOVE_INVALID (all bits set, never a legal move)."""
+    dev = _id_device(device)
+    i = _as_int_tensor(ids, torch.int32, dev)
+    out = torch.empty(i.shape, dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        N.check(N.lib.ddz_moves_of_ids(i.data_ptr(), i.numel(), out.data_ptr(), torch.cuda.current_stream(dev).cuda_stream),
+                "ddz_moves_of_ids")
+    return out
+
+
+def action_space(device=None):
+    """The whole universe of action ids: moves int64 [13551] (moves[id] = packed move), card_py_index int64 [13551] (the
+    move's index in card.py's 13 527-move action space, -1 for the 24 rocket-kicker moves card.py leaves out) and
+    id_of_card_py int64 [13527] (the inverse map)."""
+    dev = _id_device(device)
+    moves = moves_of_ids(torch.arange(N.NUM_ACTION_IDS, dtype=torch.int32, device=dev), dev)
+    c = unpack_counts(moves)
+    # the rocket-kicker extras are the only moves with both jokers among 6 (4+1+1) or 8 (two-trio 3+1 plane) cards
+    extra = (c[:, 13] == 1) & (c[:, 14] == 1) & ((c.sum(-1) == 6) | (c.sum(-1) == 8))
+    keep = ~extra
+    card_py = torch.where(keep, torch.cumsum(keep.to(torch.int64), 0) - 1, torch.full_like(moves, -1))
+    return ActionSpace(moves, card_py, keep.nonzero(as_tuple=True)[0])
 
 
 # ---------------------------------------------------------------------- B = 1 views (exact reference signatures)

@@ -43,7 +43,7 @@ extern "C" {
 #endif
 
 #define DDZ_ABI_VERSION 3   /* 3: ddz_mcts_moves, ddz_playout_pruned, ddz_q_features (+ ddz_uct_search, ddz_uct_workspace_bytes,
-                            * ddz_determinize, ddz_uct_pool, ddz_encode_face_gather:
+                            * ddz_determinize, ddz_uct_pool, ddz_encode_face_gather, ddz_move_ids, ddz_moves_of_ids, ddz_legal_mask:
                             * new entry points only, backward compatible).  2: ddz_mpipe_*, ddz_set_tile_order, ddz_prob_form; cut lists are played
                             * from their visible part */
 #define DDZ_MAX_LEGAL 512  /* upper bound of legal moves of one decision (worst known hand: 497) */
@@ -393,6 +393,38 @@ int ddz_encode_face(const void* state, int variant, float* face, int B, void* st
 #define DDZ_ROWS_CONCAT 1
 int ddz_encode_face_gather(const void* state, int variant, const int64_t* rows, int64_t n, const uint64_t* moves,
                            float* face, float* move_rows, int layout, int B, void* stream);
+
+/* Action ids: a fixed index per move, the same in every position (the reference's action space, rule_based/utils/card.py:34-159,
+ * which server/rule_utils/utils.py:21-38 get_mask_onehot60 masks).  The UNIVERSE is card.py's action_space in its order with
+ * the 24 moves r.get_moves emits beyond it -- the {black joker, red joker} kicker pair of a two-trio 3+1 plane and of a 4+1+1
+ * (server/mcts/get_moves.py:22-34) -- slotted in where card.py's combination loops would have produced them: 13 551 moves,
+ * id 0 = pass.  (The card.py index of a move is its id minus the number of those 24 below it.)  Canonical legal lists are in
+ * universe order, so the ids of a list strictly increase.  Ids do not depend on the probability form.
+ *
+ * ddz_move_ids: ids[i] = id of moves[i], -1 when moves[i] is not a move of the universe (counts no category produces, a
+ * kicker equal to a main rank, a straight through '2', a nibble above 4, ...).
+ * ddz_moves_of_ids: moves[i] = the packed move of ids[i]; an id outside [0, DDZ_NUM_ACTION_IDS) gives DDZ_MOVE_INVALID
+ * (never a legal move: ddz_step with DDZ_CHOICE_MOVE treats it as an illegal choice).
+ * n = 0 returns 0 without a launch; n < 0, or a NULL buffer with n > 0: DDZ_E_ARG before any CUDA call.
+ *
+ * ddz_legal_mask: one full row per env over the CURRENT lists (offsets / actions_u64 as ddz_observe, ddz_rollout_step or
+ * ddz_legal_moves wrote them, holding cap moves):
+ *   DDZ_MASK_BITS   out uint32 [B][DDZ_MASK_WORDS], bit (id & 31) of word (id >> 5); the 17 bits past id 13 550 are zero;
+ *                   out 16-byte aligned;
+ *   DDZ_MASK_BYTES  out uint8 [B][DDZ_NUM_ACTION_IDS], 1 for a legal id else 0 (a torch bool mask).
+ * Every byte of every row is written.  Only list entries below cap are read: an env whose list runs past cap gets the stored
+ * part and stats[7] (stats may be NULL) counts it once; a finished env (empty list) gets an all-zero row.
+ * NULL offsets / out, actions_u64 NULL with cap > 0, cap < 0, B <= 0, an unknown layout or a misaligned bits row: DDZ_E_ARG
+ * before any CUDA call. */
+#define DDZ_NUM_ACTION_IDS 13551
+#define DDZ_MOVE_INVALID 0xFFFFFFFFFFFFFFFFull
+#define DDZ_MASK_BITS 0
+#define DDZ_MASK_BYTES 1
+#define DDZ_MASK_WORDS 424          /* ceil(DDZ_NUM_ACTION_IDS / 32) */
+int ddz_move_ids(const uint64_t* moves, int64_t n, int32_t* ids, void* stream);
+int ddz_moves_of_ids(const int32_t* ids, int64_t n, uint64_t* moves, void* stream);
+int ddz_legal_mask(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, int layout, void* out, int64_t* stats,
+                   int B, void* stream);
 
 #ifdef __cplusplus
 }
