@@ -25,6 +25,7 @@
 // needs is many independent warps with stores in flight and no synchronisation.
 #include <cuda.h>
 #include <cuda_runtime.h>
+#include <cfloat>
 #include <climits>
 #include <cstdint>
 #include <cstdio>
@@ -40,6 +41,7 @@
 #include "ddz_flat.cuh"
 #include "ddz_search.cuh"
 #include "ddz_ids.cuh"
+#include "ddz_policy.cuh"
 
 namespace ddz {
 
@@ -2358,6 +2360,69 @@ int ddz_legal_mask(const int32_t* offsets, const uint64_t* actions_u64, int64_t 
     if (layout == DDZ_MASK_BITS) k_legal_mask<false><<<grid, kMaskWarps * 32, 0, st>>>(offsets, actions_u64, cap, out, stats, B);
     else k_legal_mask<true><<<grid, kMaskWarps * 32, 0, st>>>(offsets, actions_u64, cap, out, stats, B);
     DDZ_LAUNCH_CHECK("k_legal_mask");
+    return 0;
+}
+
+static bool policy_args_ok(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* logits, int dtype,
+                           int64_t ld, int B) {
+    if (!offsets || !logits || B <= 0 || cap < 0 || (cap > 0 && !actions_u64) || ld < DDZ_NUM_ACTION_IDS) return false;
+    if (dtype != DDZ_DTYPE_F32 && dtype != DDZ_DTYPE_BF16) return false;
+    return (reinterpret_cast<uintptr_t>(logits) & (dtype == DDZ_DTYPE_F32 ? 3u : 1u)) == 0;
+}
+static unsigned policy_grid(int B) { return (unsigned)((B + policy_head::kWarps - 1) / policy_head::kWarps); }
+
+int ddz_policy_sample(void* state, const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* logits,
+                      int dtype, int64_t ld, float temperature, uint64_t seed, uint64_t env0, uint32_t stepno,
+                      const uint8_t* env_mask, int32_t* choice, int32_t* ids, float* logp, float* entropy, int64_t* stats,
+                      int B, void* stream) {
+    if (!policy_args_ok(offsets, actions_u64, cap, logits, dtype, ld, B) || !choice || !ids || !logp || !entropy) return DDZ_E_ARG;
+    if (!(temperature >= 0.f) || !(temperature <= FLT_MAX)) return DDZ_E_ARG;              // NaN, negative or infinite
+    uint32_t* meta = state ? reinterpret_cast<uint32_t*>(reinterpret_cast<uint64_t*>(state) + 9 * (size_t)B) : nullptr;
+    const cudaStream_t st = (cudaStream_t)stream;
+    const unsigned grid = policy_grid(B), threads = policy_head::kWarps * 32;
+    if (dtype == DDZ_DTYPE_F32)
+        policy_head::k_policy_sample<DDZ_DTYPE_F32><<<grid, threads, 0, st>>>(offsets, actions_u64, cap, logits, ld, temperature, seed,
+                                                                              env0, stepno, env_mask, meta, choice, ids, logp,
+                                                                              entropy, stats, B);
+    else
+        policy_head::k_policy_sample<DDZ_DTYPE_BF16><<<grid, threads, 0, st>>>(offsets, actions_u64, cap, logits, ld, temperature, seed,
+                                                                               env0, stepno, env_mask, meta, choice, ids, logp,
+                                                                               entropy, stats, B);
+    DDZ_LAUNCH_CHECK("k_policy_sample");
+    return 0;
+}
+
+int ddz_policy_logprob(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* logits, int dtype,
+                       int64_t ld, const int32_t* ids, float* logp, float* entropy, float* lse, int64_t* stats, int B,
+                       void* stream) {
+    if (!policy_args_ok(offsets, actions_u64, cap, logits, dtype, ld, B) || !ids || !logp || !entropy) return DDZ_E_ARG;
+    const cudaStream_t st = (cudaStream_t)stream;
+    const unsigned grid = policy_grid(B), threads = policy_head::kWarps * 32;
+    if (dtype == DDZ_DTYPE_F32)
+        policy_head::k_policy_logprob<DDZ_DTYPE_F32><<<grid, threads, 0, st>>>(offsets, actions_u64, cap, logits, ld, ids, logp,
+                                                                               entropy, lse, stats, B);
+    else
+        policy_head::k_policy_logprob<DDZ_DTYPE_BF16><<<grid, threads, 0, st>>>(offsets, actions_u64, cap, logits, ld, ids, logp,
+                                                                                entropy, lse, stats, B);
+    DDZ_LAUNCH_CHECK("k_policy_logprob");
+    return 0;
+}
+
+int ddz_policy_logprob_backward(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* logits,
+                                int dtype, int64_t ld, const int32_t* ids, const float* lse, const float* grad_logp,
+                                const float* grad_entropy, void* grad_logits, int64_t grad_ld, int B, void* stream) {
+    if (!policy_args_ok(offsets, actions_u64, cap, logits, dtype, ld, B) || !ids || !lse || !grad_logits) return DDZ_E_ARG;
+    if (grad_ld < DDZ_NUM_ACTION_IDS || (reinterpret_cast<uintptr_t>(grad_logits) & (dtype == DDZ_DTYPE_F32 ? 3u : 1u)) != 0)
+        return DDZ_E_ARG;
+    const cudaStream_t st = (cudaStream_t)stream;
+    const unsigned grid = policy_grid(B), threads = policy_head::kWarps * 32;
+    if (dtype == DDZ_DTYPE_F32)
+        policy_head::k_policy_logprob_backward<DDZ_DTYPE_F32><<<grid, threads, 0, st>>>(
+            offsets, actions_u64, cap, logits, ld, ids, lse, grad_logp, grad_entropy, grad_logits, grad_ld, B);
+    else
+        policy_head::k_policy_logprob_backward<DDZ_DTYPE_BF16><<<grid, threads, 0, st>>>(
+            offsets, actions_u64, cap, logits, ld, ids, lse, grad_logp, grad_entropy, grad_logits, grad_ld, B);
+    DDZ_LAUNCH_CHECK("k_policy_logprob_backward");
     return 0;
 }
 

@@ -15,6 +15,7 @@ import numpy as np
 import torch
 
 from . import _native as N
+from .policy import _sample as _policy_sample
 from .deals import DEAL_SEED0, default_deals, random_deals, adversarial_pairs, ADVERSARIAL_POOL  # noqa: F401  (re-exported)
 
 VARIANT_CHANNELS = (4, 7, 9, 6)
@@ -351,6 +352,14 @@ class BatchedEnv:
         not legal in its env, or outside [0, 13551), is an illegal choice: the env is left as it is, its sticky error bit
         is set, stats[7] counts it, and debug=True raises."""
         return self._step(moves_of_ids(self._to_dev(ids, torch.int32), self.device), N.CHOICE_MOVE)
+
+    def step_policy(self, logits, temperature=1.0, seed=0):
+        """A fixed-head policy's decision in one call: policy_sample(self, logits, temperature, seed), then step(choice).
+        Returns ((r, done, cat), (choice, ids, logp, entropy)).  The stepped state is the one step_ids(ids) reaches.  An env
+        whose legal logits give nothing to draw from gets choice -1, which the step treats as an illegal choice (sticky error
+        bit, counted once in stats[7])."""
+        sample = _policy_sample(self, logits, temperature, seed, None, record=False)
+        return self._step(sample[0], N.CHOICE_INDEX), sample
 
     def step_manual(self, onehot_cards):
         """envi.py:63-70: onehot float/int [B,15,4] (a row of valid_actions per env) -> (r, done, cat)."""

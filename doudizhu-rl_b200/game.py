@@ -21,6 +21,7 @@ import torch
 
 from .agent import BatchedGreedyPolicy
 from .env import VARIANT_CHANNELS, random_deals
+from .policy import _sample as policy_sample
 from .trainer import PackedReplayBuffer, ReplayBuffer, TransitionCollector, td_step
 
 # config.py:7-14
@@ -105,15 +106,18 @@ class BatchedGame:
     `dqns_dict[role]` is called as `dqn_cls(net_cls, face_channels, device)` (BatchedDQN's signature).
     search_dict (optional) seats the search bot: role -> keyword arguments of search.pimc_search, e.g.
     {"lord": {"determinizations": 8, "computation_budget": 125}}; that role plays from its own view (determinized UCT),
-    or with "determinizations": 0 the full-information search.uct_search, which sees every hand.  A role has a net or a
-    search entry, not both.
+    or with "determinizations": 0 the full-information search.uct_search, which sees every hand.
+    policy_dict (optional) seats a fixed-head policy: role -> a module (on the game's device) that maps the env's face
+    [B, C, 15, 4] to logits [B, 13551] over the action ids; that role samples its move from the softmax over its legal ids
+    (policy.policy_sample) at temperature `policy_temperature` (1.0; compete plays 0, the argmax).  Learning stays with the
+    caller.  A role has a net, a search entry or a policy entry, never two.
     replay="packed" keeps the learning roles' transitions as packed states and moves (trainer.PackedReplayBuffer, 176 B a
     transition instead of 2 * 240 * (C + 1) + 8 B): `dqns_dict[role]` is then called with the extra keyword replay="packed".
     Set the capacity through the DQN class, e.g. functools.partial(BatchedDQN, replay_size=10_000_000)."""
 
     def __init__(self, env_cls, nets_dict, dqns_dict, reward_dict=None, train_dict=None, preload=None, seed=None,
                  debug=False, num_envs=4096, pool_games=8, deals=None, device=None, updates_per_step=1, search_dict=None,
-                 replay="float"):
+                 replay="float", policy_dict=None):
         if reward_dict is None:
             reward_dict = {"lord": 100, "down": 50, "up": 50}
         if train_dict is None:
@@ -129,6 +133,13 @@ class BatchedGame:
                 raise ValueError("unknown role %r in search_dict" % (role,))
             if nets_dict.get(role):
                 raise ValueError("role %r has both a net and a search entry" % (role,))
+        self.policy_dict = dict(policy_dict or {})
+        for role in self.policy_dict:
+            if role not in ROLE_INDEX:
+                raise ValueError("unknown role %r in policy_dict" % (role,))
+            if nets_dict.get(role) or role in self.search_dict:
+                raise ValueError("role %r has a policy entry and a net or search entry" % (role,))
+        self.policy_temperature = 1.0
         self._search_seed = int(seed) if seed else 0
         self.env = env_cls(num_envs, debug=debug, seed=seed, device=device)
         self.B, self.device = self.env.B, self.env.device
@@ -232,6 +243,14 @@ class BatchedGame:
             mine = (seat == ROLE_INDEX[role]) & live
             if bool(mine.any()):
                 choice = torch.where(mine, self._search(kw, mine).to(torch.int64).clamp(min=0), choice)
+        for role, module in self.policy_dict.items():
+            mine = (seat == ROLE_INDEX[role]) & live
+            if bool(mine.any()):
+                with torch.no_grad():
+                    logits = module(env.face)
+                # record=False: a -1 (nothing to draw from) is counted once, as the step's illegal choice
+                k = policy_sample(env, logits, self.policy_temperature, self._search_seed, mine, record=False)[0]
+                choice = torch.where(mine, k.to(torch.int64), choice)
         was_done = env.is_done.clone()
         env.step(choice.to(torch.int32))
         env.observe()
@@ -316,14 +335,15 @@ class BatchedGame:
     # ------------------------------------------------------------------ evaluation (game.py:240-275)
     @staticmethod
     def compete(env_cls, nets_dict, dqns_dict, model_dict, total=1000, print_every=100, debug=True, num_envs=4096,
-                seed=None, device=None, nets=None, search_dict=None):
+                seed=None, device=None, nets=None, search_dict=None, policy_dict=None):
         """greedy play of the given networks (others random) until `total` games have ended; Counter of wins per role.
         `nets` may hand over already constructed networks per role instead of checkpoints in model_dict; search_dict
-        seats the search bot as in BatchedGame."""
+        seats the search bot and policy_dict a fixed-head policy as in BatchedGame (played at temperature 0: argmax)."""
         assert not (nets_dict.keys() ^ dqns_dict.keys()), "Net and DQN must match"
         train_dict = {r: False for r in ROLES}
         game = BatchedGame(env_cls, nets_dict, dqns_dict, train_dict=train_dict, preload=model_dict or {}, seed=seed,
-                           debug=False, num_envs=num_envs, device=device, search_dict=search_dict)
+                           debug=False, num_envs=num_envs, device=device, search_dict=search_dict, policy_dict=policy_dict)
+        game.policy_temperature = 0.0
         for role, net in (nets or {}).items():
             getattr(game, role).policy_net.load_state_dict(net.state_dict())
         wins = collections.Counter()

@@ -43,7 +43,8 @@ extern "C" {
 #endif
 
 #define DDZ_ABI_VERSION 3   /* 3: ddz_mcts_moves, ddz_playout_pruned, ddz_q_features (+ ddz_uct_search, ddz_uct_workspace_bytes,
-                            * ddz_determinize, ddz_uct_pool, ddz_encode_face_gather, ddz_move_ids, ddz_moves_of_ids, ddz_legal_mask:
+                            * ddz_determinize, ddz_uct_pool, ddz_encode_face_gather, ddz_move_ids, ddz_moves_of_ids, ddz_legal_mask,
+                            * ddz_policy_sample, ddz_policy_logprob, ddz_policy_logprob_backward:
                             * new entry points only, backward compatible).  2: ddz_mpipe_*, ddz_set_tile_order, ddz_prob_form; cut lists are played
                             * from their visible part */
 #define DDZ_MAX_LEGAL 512  /* upper bound of legal moves of one decision (worst known hand: 497) */
@@ -425,6 +426,60 @@ int ddz_move_ids(const uint64_t* moves, int64_t n, int32_t* ids, void* stream);
 int ddz_moves_of_ids(const int32_t* ids, int64_t n, uint64_t* moves, void* stream);
 int ddz_legal_mask(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, int layout, void* out, int64_t* stats,
                    int B, void* stream);
+
+/* Fixed-head policies: a softmax over an output head of DDZ_NUM_ACTION_IDS logits per env, restricted to the env's legal
+ * ids, without a dense mask.  logits: row b at logits + b * ld elements (ld >= DDZ_NUM_ACTION_IDS), entry id = the logit of
+ * action id `id`; dtype DDZ_DTYPE_F32 (float) or DDZ_DTYPE_BF16 (bfloat16, widened exactly to float).  The lists are the
+ * CURRENT ones (offsets / actions_u64 holding cap moves, as for ddz_legal_mask) and must be complete: an env whose list was
+ * cut or dropped by the capacity is not scored (below) and is counted in stats[7] (stats may be NULL); nothing past cap is
+ * read.  One warp per env reads only the logits of its legal ids.  All arithmetic is float.  With m = the largest legal
+ * logit, T the temperature, z_i = (l_i - m) / T and w_i = expf(z_i) over the env's list i = 0 .. N-1 (canonical order =
+ * increasing id):
+ *   R_i = the running sum of the w_i in this order: 32-entry chunks in list order; within a chunk the lanes' inclusive scan
+ *         (step d = 1, 2, 4, 8, 16: lane k >= d adds the value of lane k - d; lanes past the list hold 0), added to R at
+ *         lane 31 of the chunk before;
+ *   S   = R_j of the LAST entry j with w_j > 0 (NaN when no entry has w > 0 or a legal logit is NaN);
+ *   p_i = w_i / S,  log p_i = z_i - logf(S),  H = logf(S) - (sum of w_i z_i over w_i > 0) / S.
+ *
+ * ddz_policy_sample: one move per env.  temperature > 0: u = (philox(seed, env0 + b, stepno) >> 8) * 2^-24 (the key and
+ * counter of the DDZ_CHOICE_PHILOX stream, in the 24-bit form of ddz_select_actions' exploration draw), and the chosen
+ * entry is the first i with w_i > 0 and R_i > u * S (float product).  u * S < S = R_j, so entry j always qualifies: a
+ * list with a finite S always gets an entry, and never one of probability 0.  temperature = 0: argmax, the first entry
+ * (lowest id) of the largest logit, a NaN beating every number as in torch.argmax; logp and entropy are those of T = 1.
+ * Outputs int32 choice[B] (the index in the env's list: feed ddz_step with DDZ_CHOICE_INDEX), int32 ids[B], float logp[B]
+ * (log p of the chosen entry), float entropy[B] (H).  Finished envs and masked-out envs (env_mask uint8[B], NULL = all)
+ * get choice = ids = -1, logp = entropy = 0, and are no error.  Nothing is drawn when the legal logits are all -inf, or, at
+ * temperature > 0, one of them is NaN or +inf (no finite positive S): -1 / -1 / 0 / 0, stats[7] counts the env once and,
+ * when state != NULL, its sticky error bit (meta bit 5) is set.  A cut or dropped list gives -1 / -1 / 0 / 0 and stats[7]
+ * (no sticky bit: the capacity, not the env, is at fault).
+ *
+ * ddz_policy_logprob (training forward, T = 1): for the chosen ids[b] (e.g. from replay), logp[b] = log p of that id,
+ * entropy[b] = H, and lse[b] (optional, for the backward) = m + logf(S).  An id not in the env's list gives logp = -inf and
+ * is counted in stats[7].  Legal logits with no softmax (all -inf, or a NaN or +inf among them: S = NaN) give NaN in all
+ * three, as torch's log_softmax does, and are counted in stats[7] (once per env).  An env with an empty list gives
+ * logp = entropy = 0 and lse = -inf; a cut or dropped list gives NaN in all three and stats[7].
+ *
+ * ddz_policy_logprob_backward: the full gradient row of every env, grad_logits [B][grad_ld] (the first DDZ_NUM_ACTION_IDS
+ * elements of a row are written, once each, in 16-byte pieces; the padding is not touched) in the dtype of the logits:
+ *   g_lp (1[id = ids[b]] - p_id) - g_ent p_id (log p_id + H)   on the legal ids, with p_id = expf(l_id - lse[b]),
+ *   exactly 0 on every other id, and on the whole row of an env with an empty, cut or dropped list;
+ * H is recomputed as -sum p log p; g_lp = grad_logp[b], g_ent = grad_entropy[b] (either may be NULL = 0).
+ *
+ * NULL offsets / logits / outputs, actions_u64 NULL with cap > 0, cap < 0, B <= 0, ld or grad_ld < DDZ_NUM_ACTION_IDS, an
+ * unknown dtype, a logits or grad row pointer not aligned to its element, or a temperature that is negative, NaN or
+ * infinite: DDZ_E_ARG before any CUDA call. */
+#define DDZ_DTYPE_F32 0
+#define DDZ_DTYPE_BF16 1
+int ddz_policy_sample(void* state, const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* logits,
+                      int dtype, int64_t ld, float temperature, uint64_t seed, uint64_t env0, uint32_t stepno,
+                      const uint8_t* env_mask, int32_t* choice, int32_t* ids, float* logp, float* entropy, int64_t* stats,
+                      int B, void* stream);
+int ddz_policy_logprob(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* logits, int dtype,
+                       int64_t ld, const int32_t* ids, float* logp, float* entropy, float* lse, int64_t* stats, int B,
+                       void* stream);
+int ddz_policy_logprob_backward(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* logits,
+                                int dtype, int64_t ld, const int32_t* ids, const float* lse, const float* grad_logp,
+                                const float* grad_entropy, void* grad_logits, int64_t grad_ld, int B, void* stream);
 
 #ifdef __cplusplus
 }
