@@ -337,10 +337,9 @@ struct __align__(128) WarpSmem {
     float4 lut[kLutEntries];
 };
 
-// V: face variant or -1 (no face).  MODE: see enum Mode.
+// V: face variant or -1 (no face).  MODE: see enum Mode.  The body of k_env and of lean::k_step_observe.
 template <int V, int MODE>
-__global__ void __launch_bounds__(kThreads, kMinCtasPerSm) k_env(void* state, StepArgs a, OutArgs o,
-                                                  Workspace ws, int64_t* stats, int B) {
+DDZ_DEV void env_kernel(void* state, const StepArgs& a, const OutArgs& o, const Workspace& ws, int64_t* stats, int B) {
     constexpr bool STEP = (MODE == kStepOnly || MODE == kStepObserve);
     constexpr bool EMIT = (MODE != kStepOnly);
     constexpr int C = FaceCfg<(V < 0 ? 0 : V)>::C;
@@ -553,6 +552,27 @@ __global__ void __launch_bounds__(kThreads, kMinCtasPerSm) k_env(void* state, St
         }
     }
 }
+template <int V, int MODE>
+__global__ void __launch_bounds__(kThreads, kMinCtasPerSm) k_env(void* state, StepArgs a, OutArgs o,
+                                                  Workspace ws, int64_t* stats, int B) {
+    env_kernel<V, MODE>(state, a, o, ws, stats, B);
+}
+
+// The fused step with a face (ddz_rollout_step) at fewer resident warps: 16 per SM leave 110 registers to a warp, where
+// k_env's 28 (one wave of 131 072 envs) leave 72 and spill.  The store stream does not need more warps than that: with
+// four env groups of 32 768 envs in flight (bench.py config 4) the step is 5-6 % faster on a B200, 24 / 20 warps per SM
+// give 3 % (profiles/r10_lean_step.json).  A launch whose grid does not fit at once at this occupancy runs k_env.
+namespace lean {
+#ifndef DDZ_LEAN_WARPS_PER_SM
+#define DDZ_LEAN_WARPS_PER_SM 16
+#endif
+constexpr int kMinCtas = DDZ_LEAN_WARPS_PER_SM / kWarpsPerCta;
+template <int V>
+__global__ void __launch_bounds__(kThreads, kMinCtas) k_step_observe(void* state, StepArgs a, OutArgs o, Workspace ws,
+                                                                     int64_t* stats, int B) {
+    env_kernel<V, kStepObserve>(state, a, o, ws, stats, B);
+}
+}  // namespace lean
 
 // ------------------------------------------------------------------------------------------------
 // r.get_moves for n independent (hand, last) pairs, long lists welcome (ddz_legal_moves; BASELINE config 5).
@@ -1600,31 +1620,53 @@ static int cuda_fail(cudaError_t e, const char* what) {
         if (e_ != cudaSuccess) return cuda_fail(e_, what);             \
     } while (0)
 
-template <int V, int MODE>
-static int launch_env(void* state, const StepArgs& a, const OutArgs& o, void* workspace, int64_t* stats, int B, cudaStream_t st) {
-    const size_t smem = (MODE == kStepOnly) ? 0 : kWarpsPerCta * sizeof(WarpSmem);
-    Workspace ws = workspace ? ws_of(workspace) : Workspace{nullptr, nullptr};
-    const int grid = (ntiles(B) + kWarpsPerCta - 1) / kWarpsPerCta;
-    // CTAs of this instantiation that fit on the device at once, per device (the shapes of the devices of a box may differ)
+// CTAs of `kernel` (instantiation V, MODE, LEAN) that fit on the current device at once, cached per device (the shapes of
+// the devices of a box may differ)
+template <int V, int MODE, bool LEAN>
+static int resident_ctas(const void* kernel, size_t smem, int& resident) {
     static std::atomic<int> resident_of[64];
     static std::once_flag once;
     std::call_once(once, [] { for (auto& r : resident_of) r.store(-1); });
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) return cuda_fail(cudaGetLastError(), "cudaGetDevice");
-    int resident = dev < 64 ? resident_of[dev].load(std::memory_order_relaxed) : -1;
+    resident = dev < 64 ? resident_of[dev].load(std::memory_order_relaxed) : -1;
     if (resident < 0) {
         int per_sm = 0, sms = 0;
         if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_env<V, MODE>, kThreads, smem) != cudaSuccess)
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, smem) != cudaSuccess)
             return cuda_fail(cudaGetLastError(), "occupancy query");
         resident = per_sm * sms;
         if (dev < 64) resident_of[dev].store(resident, std::memory_order_relaxed);
+    }
+    return 0;
+}
+template <int V, int MODE>
+static int launch_env(void* state, const StepArgs& a, const OutArgs& o, void* workspace, int64_t* stats, int B, cudaStream_t st) {
+    const size_t smem = (MODE == kStepOnly) ? 0 : kWarpsPerCta * sizeof(WarpSmem);
+    Workspace ws = workspace ? ws_of(workspace) : Workspace{nullptr, nullptr};
+    const int grid = (ntiles(B) + kWarpsPerCta - 1) / kWarpsPerCta;
+    int resident = 0;
+    if (int rc = resident_ctas<V, MODE, false>((const void*)k_env<V, MODE>, smem, resident)) return rc;
+    // a step with a face whose grid fits at once at lean::k_step_observe's occupancy runs that kernel (more registers
+    // per warp, no spills); a larger one runs k_env, which holds one wave of 131 072 envs
+    bool lean_fits = false;
+    if constexpr (MODE == kStepObserve && V >= 0) {
+        int lean_resident = 0;
+        if (int rc = resident_ctas<V, MODE, true>((const void*)lean::k_step_observe<V>, smem, lean_resident)) return rc;
+        if (grid <= lean_resident) { lean_fits = true; resident = lean_resident; }
     }
     OutArgs oo = o;
     // tile = launch position needs every lower tile to be running or done when a tile waits on it: true when the whole grid
     // is resident at once (and CTAs are dispatched in launch order, as they are in practice).  A caller whose other kernels
     // share the GPU asks for tickets instead (ddz_set_tile_order): correct under any dispatch order.
     oo.static_tiles = (g_tile_order.load(std::memory_order_relaxed) == DDZ_TILES_AUTO && grid <= resident) ? 1 : 0;
+    if constexpr (MODE == kStepObserve && V >= 0) {
+        if (lean_fits) {
+            lean::k_step_observe<V><<<grid, kThreads, smem, st>>>(state, a, oo, ws, stats, B);
+            DDZ_LAUNCH_CHECK("lean::k_step_observe");
+            return 0;
+        }
+    }
     k_env<V, MODE><<<grid, kThreads, smem, st>>>(state, a, oo, ws, stats, B);
     DDZ_LAUNCH_CHECK("k_env");
     return 0;
