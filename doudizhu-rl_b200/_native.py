@@ -28,7 +28,9 @@ EXPORTS = ("ddz_abi_version", "ddz_prob_form", "ddz_set_tile_order", "ddz_face_c
            "ddz_mpipe_create", "ddz_mpipe_destroy", "ddz_mpipe_step", "ddz_mpipe_wait", "ddz_mpipe_refill", "ddz_mpipe_flush", "ddz_mpipe_join",
            "ddz_mcts_moves", "ddz_playout_pruned", "ddz_q_features", "ddz_uct_workspace_bytes", "ddz_uct_search",
            "ddz_determinize", "ddz_uct_pool", "ddz_encode_face_gather", "ddz_move_ids", "ddz_moves_of_ids", "ddz_legal_mask",
-           "ddz_policy_sample", "ddz_policy_logprob", "ddz_policy_logprob_backward")
+           "ddz_policy_sample", "ddz_policy_logprob", "ddz_policy_logprob_backward", "ddz_policy_linear_logits",
+           "ddz_policy_linear_sample", "ddz_policy_linear_logprob", "ddz_policy_linear_backward",
+           "ddz_policy_linear_workspace_bytes", "ddz_policy_linear_grad_weight")
 
 lib = C.CDLL(LIB_PATH)
 _missing = [name for name in EXPORTS if not hasattr(lib, name)]
@@ -128,6 +130,16 @@ lib.ddz_policy_sample.argtypes = [_vp, _vp, _vp, _i64, _vp, _i, _i64, C.c_float,
 lib.ddz_policy_logprob.argtypes = [_vp, _vp, _i64, _vp, _i, _i64, _vp, _vp, _vp, _vp, _vp, _i, _vp]
 lib.ddz_policy_logprob_backward.argtypes = [_vp, _vp, _i64, _vp, _i, _i64, _vp, _vp, _vp, _vp, _vp, _i64, _i, _vp]
 DTYPE_F32, DTYPE_BF16 = 0, 1
+lib.ddz_policy_linear_logits.argtypes = [_vp, _vp, _i64, _vp, _vp, _vp, _i, _i, _i64, _vp, _vp, _i, _vp]
+lib.ddz_policy_linear_sample.argtypes = [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _i, _i, _i64, C.c_float, _u64, _u64, _u32, _vp,
+                                         _vp, _vp, _vp, _vp, _vp, _i, _vp]
+lib.ddz_policy_linear_logprob.argtypes = [_vp, _vp, _i64, _vp, _vp, _vp, _i, _i, _i64, _vp, _vp, _vp, _vp, _vp, _i, _vp]
+lib.ddz_policy_linear_backward.argtypes = [_vp, _vp, _i64, _vp, _vp, _vp, _i, _i, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i64,
+                                           _i, _vp]
+lib.ddz_policy_linear_workspace_bytes.argtypes = [_i64, _i]
+lib.ddz_policy_linear_workspace_bytes.restype = C.c_size_t
+lib.ddz_policy_linear_grad_weight.argtypes = [_vp, _i64, _vp, _i, _i, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp]
+LINEAR_MAX_HIDDEN = 1024
 
 if lib.ddz_abi_version() != ABI_VERSION:
     raise ImportError("libddz_b200.so ABI %d != binding %d: rebuild" % (lib.ddz_abi_version(), ABI_VERSION))

@@ -33,6 +33,7 @@
 #include <cstring>
 #include <atomic>
 #include <mutex>
+#include <type_traits>
 
 #include "../../include/ddz_b200.h"
 #include "ddz_device.cuh"
@@ -42,6 +43,7 @@
 #include "ddz_search.cuh"
 #include "ddz_ids.cuh"
 #include "ddz_policy.cuh"
+#include "ddz_policy_linear.cuh"
 
 namespace ddz {
 
@@ -1749,6 +1751,14 @@ static int launch_face_gather(const void* state, const int64_t* rows, int64_t n,
     return 0;
 }
 
+// f(std::integral_constant<int, DT>) for the dtype code of a linear head
+template <class F>
+static void by_dtype(int dtype, F&& f) {
+    if (dtype == DDZ_DTYPE_F32) f(std::integral_constant<int, DDZ_DTYPE_F32>{});
+    else f(std::integral_constant<int, DDZ_DTYPE_BF16>{});
+}
+constexpr unsigned kLinearThreads = linear_head::kWarps * 32;
+
 extern "C" {
 
 #ifdef DDZ_TRACE
@@ -2465,6 +2475,116 @@ int ddz_policy_logprob_backward(const int32_t* offsets, const uint64_t* actions_
         policy_head::k_policy_logprob_backward<DDZ_DTYPE_BF16><<<grid, threads, 0, st>>>(
             offsets, actions_u64, cap, logits, ld, ids, lse, grad_logp, grad_entropy, grad_logits, grad_ld, B);
     DDZ_LAUNCH_CHECK("k_policy_logprob_backward");
+    return 0;
+}
+
+// linear heads: hidden / weight (16-byte rows, H and ld whole 16-byte pieces, H <= 1024) and bias (element-aligned) of one dtype
+static bool linear_head_ok(const void* hidden, const void* weight, const void* bias, int dtype, int H, int64_t ld) {
+    if (!hidden || !weight || (dtype != DDZ_DTYPE_F32 && dtype != DDZ_DTYPE_BF16)) return false;
+    const int esz = dtype == DDZ_DTYPE_F32 ? 4 : 2, vec = 16 / esz;
+    if (H <= 0 || H > linear_head::kMaxHidden || H % vec != 0 || ld < H || ld % vec != 0) return false;
+    return ((reinterpret_cast<uintptr_t>(hidden) | reinterpret_cast<uintptr_t>(weight)) & 15u) == 0 &&
+           (reinterpret_cast<uintptr_t>(bias) & (uintptr_t)(esz - 1)) == 0;
+}
+static bool linear_args_ok(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* hidden,
+                           const void* weight, const void* bias, int dtype, int H, int64_t ld, int B) {
+    if (!offsets || B <= 0 || cap < 0 || (cap > 0 && !actions_u64)) return false;
+    return linear_head_ok(hidden, weight, bias, dtype, H, ld);
+}
+
+int ddz_policy_linear_logits(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* hidden,
+                             const void* weight, const void* bias, int dtype, int H, int64_t ld, float* out, int64_t* stats,
+                             int B, void* stream) {
+    if (!linear_args_ok(offsets, actions_u64, cap, hidden, weight, bias, dtype, H, ld, B) || (cap > 0 && !out)) return DDZ_E_ARG;
+    by_dtype(dtype, [&](auto dt) {
+        constexpr int DT = decltype(dt)::value;
+        linear_head::k_linear_logits<DT><<<policy_grid(B), kLinearThreads, 0, (cudaStream_t)stream>>>(
+            offsets, actions_u64, cap, linear_head::Head<DT>{hidden, weight, bias, H, ld}, out, stats, B);
+    });
+    DDZ_LAUNCH_CHECK("k_linear_logits");
+    return 0;
+}
+
+int ddz_policy_linear_sample(void* state, const int32_t* offsets, const uint64_t* actions_u64, int64_t cap,
+                             const void* hidden, const void* weight, const void* bias, int dtype, int H, int64_t ld,
+                             float temperature, uint64_t seed, uint64_t env0, uint32_t stepno, const uint8_t* env_mask,
+                             int32_t* choice, int32_t* ids, float* logp, float* entropy, int64_t* stats, int B, void* stream) {
+    if (!linear_args_ok(offsets, actions_u64, cap, hidden, weight, bias, dtype, H, ld, B) || !choice || !ids || !logp ||
+        !entropy)
+        return DDZ_E_ARG;
+    if (!(temperature >= 0.f) || !(temperature <= FLT_MAX)) return DDZ_E_ARG;              // NaN, negative or infinite
+    uint32_t* meta = state ? reinterpret_cast<uint32_t*>(reinterpret_cast<uint64_t*>(state) + 9 * (size_t)B) : nullptr;
+    by_dtype(dtype, [&](auto dt) {
+        constexpr int DT = decltype(dt)::value;
+        linear_head::k_linear_sample<DT><<<policy_grid(B), kLinearThreads, 0, (cudaStream_t)stream>>>(
+            offsets, actions_u64, cap, linear_head::Head<DT>{hidden, weight, bias, H, ld}, temperature, seed, env0, stepno,
+            env_mask, meta, choice, ids, logp, entropy, stats, B);
+    });
+    DDZ_LAUNCH_CHECK("k_linear_sample");
+    return 0;
+}
+
+int ddz_policy_linear_logprob(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* hidden,
+                              const void* weight, const void* bias, int dtype, int H, int64_t ld, const int32_t* ids,
+                              float* logp, float* entropy, float* lse, int64_t* stats, int B, void* stream) {
+    if (!linear_args_ok(offsets, actions_u64, cap, hidden, weight, bias, dtype, H, ld, B) || !ids || !logp || !entropy)
+        return DDZ_E_ARG;
+    by_dtype(dtype, [&](auto dt) {
+        constexpr int DT = decltype(dt)::value;
+        linear_head::k_linear_logprob<DT><<<policy_grid(B), kLinearThreads, 0, (cudaStream_t)stream>>>(
+            offsets, actions_u64, cap, linear_head::Head<DT>{hidden, weight, bias, H, ld}, ids, logp, entropy, lse, stats, B);
+    });
+    DDZ_LAUNCH_CHECK("k_linear_logprob");
+    return 0;
+}
+
+int ddz_policy_linear_backward(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* hidden,
+                               const void* weight, const void* bias, int dtype, int H, int64_t ld, const int32_t* ids,
+                               const float* lse, const float* grad_logp, const float* grad_entropy, float* grad_legal,
+                               void* grad_hidden, int64_t ld_g, int B, void* stream) {
+    if (!linear_args_ok(offsets, actions_u64, cap, hidden, weight, bias, dtype, H, ld, B) || !ids || !lse || !grad_hidden ||
+        (cap > 0 && !grad_legal))
+        return DDZ_E_ARG;
+    if (ld_g < H || ld_g % (dtype == DDZ_DTYPE_F32 ? 4 : 8) != 0 || (reinterpret_cast<uintptr_t>(grad_hidden) & 15u) != 0)
+        return DDZ_E_ARG;
+    by_dtype(dtype, [&](auto dt) {
+        constexpr int DT = decltype(dt)::value;
+        linear_head::k_linear_backward<DT><<<policy_grid(B), kLinearThreads, 0, (cudaStream_t)stream>>>(
+            offsets, actions_u64, cap, linear_head::Head<DT>{hidden, weight, bias, H, ld}, ids, lse, grad_logp, grad_entropy,
+            grad_legal, grad_hidden, ld_g, B);
+    });
+    DDZ_LAUNCH_CHECK("k_linear_backward");
+    return 0;
+}
+
+size_t ddz_policy_linear_workspace_bytes(int64_t n, int H) {
+    if (n <= 0 || H <= 0 || H > linear_head::kMaxHidden) return 0;
+    const int64_t chunks = (n + linear_head::kChunk - 1) / linear_head::kChunk;
+    return (size_t)chunks * 2 * ((size_t)H + 4) * sizeof(float);
+}
+
+int ddz_policy_linear_grad_weight(const int32_t* offsets, int64_t n, const void* hidden, int dtype, int H, int64_t ld,
+                                  const float* grad_legal, const int32_t* order, const int32_t* id_offsets,
+                                  void* grad_weight, void* grad_bias, void* workspace, int B, void* stream) {
+    if (!offsets || B <= 0 || n < 0 || !grad_weight) return DDZ_E_ARG;
+    if (n > 0 && (!grad_legal || !order || !id_offsets || !workspace)) return DDZ_E_ARG;
+    if (!linear_head_ok(hidden, grad_weight, grad_bias, dtype, H, ld) || (reinterpret_cast<uintptr_t>(workspace) & 15u) != 0)
+        return DDZ_E_ARG;
+    const int64_t per_cta = (int64_t)linear_head::kChunk * linear_head::kWarps;
+    float* ws = reinterpret_cast<float*>(workspace);
+    by_dtype(dtype, [&](auto dt) {
+        constexpr int DT = decltype(dt)::value;
+        const cudaStream_t st = (cudaStream_t)stream;
+        // the head's weight and bias are not read: the id of every entry comes from id_offsets
+        const linear_head::Head<DT> hd{hidden, nullptr, nullptr, H, ld};
+        if (n > 0)
+            linear_head::k_linear_grad_chunks<DT><<<(unsigned)((n + per_cta - 1) / per_cta), kLinearThreads, 0, st>>>(
+                offsets, B, n, hd, grad_legal, order, id_offsets, grad_weight, grad_bias, ws);
+        linear_head::k_linear_grad_combine<DT><<<(DDZ_NUM_ACTION_IDS + linear_head::kWarps - 1) / linear_head::kWarps,
+                                                 kLinearThreads, 0, st>>>(H, n > 0 ? id_offsets : nullptr, grad_weight,
+                                                                          grad_bias, ws);
+    });
+    DDZ_LAUNCH_CHECK("k_linear_grad_chunks / k_linear_grad_combine");
     return 0;
 }
 

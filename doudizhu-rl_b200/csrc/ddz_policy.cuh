@@ -94,21 +94,25 @@ DDZ_DEV bool argmax_before(float va, int ia, float vb, int ib) {
     return ia < ib;
 }
 
+// The legal logits of a dense head: logits[b * ld + id].  A logit source gathers the ids and logits of env b's n entries
+// into shared memory as gather_logits does; the bodies below take any source, so that a head which computes its legal
+// logits (ddz_policy_linear.cuh) samples, scores and differentiates with the same float32 arithmetic as the dense one.
 template <int DT>
-__global__ void __launch_bounds__(kWarps * 32) k_policy_sample(const int32_t* __restrict__ offsets,
-                                                               const uint64_t* __restrict__ actions, long long cap,
-                                                               const void* __restrict__ logits, long long ld, float T,
-                                                               uint64_t seed, uint64_t env0, uint32_t stepno,
-                                                               const uint8_t* __restrict__ env_mask, uint32_t* meta,
-                                                               int32_t* choice, int32_t* ids_out, float* logp_out,
-                                                               float* entropy_out, int64_t* stats, int B) {
-    __shared__ int16_t sids[kWarps][DDZ_MAX_LEGAL];
-    __shared__ float slog[kWarps][DDZ_MAX_LEGAL];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int b = blockIdx.x * kWarps + w;
-    if (b >= B) return;
-    int16_t* ids = sids[w];
-    float* l = slog[w];
+struct DenseLogits {
+    const void* logits;
+    long long ld;
+    DDZ_DEV float gather(const uint64_t* actions, long long lo, int n, int b, int16_t* ids, float* l, int lane,
+                         bool& any_nan) const {
+        return gather_logits<DT>(actions, lo, n, logits, (size_t)b * (size_t)ld, ids, l, lane, any_nan);
+    }
+};
+
+// ddz_policy_sample of env b (one warp; ids / l: the warp's DDZ_MAX_LEGAL entries of shared memory)
+template <class Src>
+DDZ_DEV void sample_env(const Src& src, int b, int lane, const int32_t* __restrict__ offsets,
+                        const uint64_t* __restrict__ actions, long long cap, float T, uint64_t seed, uint64_t env0,
+                        uint32_t stepno, const uint8_t* __restrict__ env_mask, uint32_t* meta, int32_t* choice,
+                        int32_t* ids_out, float* logp_out, float* entropy_out, int64_t* stats, int16_t* ids, float* l) {
     int c = -1;
     float lp = 0.f, h = 0.f;
     bool cut = false, bad = false;
@@ -118,7 +122,7 @@ __global__ void __launch_bounds__(kWarps * 32) k_policy_sample(const int32_t* __
         cut = e.n < 0;
         if (!cut) {
             bool nan;
-            const float m = gather_logits<DT>(actions, e.lo, e.n, logits, (size_t)b * (size_t)ld, ids, l, lane, nan);
+            const float m = src.gather(actions, e.lo, e.n, b, ids, l, lane, nan);
             const float Te = T > 0.f ? T : 1.f;
             // no draw without a finite positive total: all legal logits -inf, or (T > 0) a NaN or +inf among them
             bad = (m == -CUDART_INF_F && !nan) || (T > 0.f && (nan || m == CUDART_INF_F));
@@ -173,8 +177,60 @@ __global__ void __launch_bounds__(kWarps * 32) k_policy_sample(const int32_t* __
     }
 }
 
-// Training forward: log-probability of the chosen ids[b] and entropy under the legal-restricted softmax (T = 1), and the
-// log-sum-exp over the legal set for the backward.
+template <int DT>
+__global__ void __launch_bounds__(kWarps * 32) k_policy_sample(const int32_t* __restrict__ offsets,
+                                                               const uint64_t* __restrict__ actions, long long cap,
+                                                               const void* __restrict__ logits, long long ld, float T,
+                                                               uint64_t seed, uint64_t env0, uint32_t stepno,
+                                                               const uint8_t* __restrict__ env_mask, uint32_t* meta,
+                                                               int32_t* choice, int32_t* ids_out, float* logp_out,
+                                                               float* entropy_out, int64_t* stats, int B) {
+    __shared__ int16_t sids[kWarps][DDZ_MAX_LEGAL];
+    __shared__ float slog[kWarps][DDZ_MAX_LEGAL];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int b = blockIdx.x * kWarps + w;
+    if (b >= B) return;
+    sample_env(DenseLogits<DT>{logits, ld}, b, lane, offsets, actions, cap, T, seed, env0, stepno, env_mask, meta, choice,
+               ids_out, logp_out, entropy_out, stats, sids[w], slog[w]);
+}
+
+// Training forward of env b: log-probability of the chosen ids[b] and entropy under the legal-restricted softmax (T = 1),
+// and the log-sum-exp over the legal set for the backward.
+template <class Src>
+DDZ_DEV void logprob_env(const Src& src, int b, int lane, const int32_t* __restrict__ offsets,
+                         const uint64_t* __restrict__ actions, long long cap, const int32_t* __restrict__ chosen,
+                         float* logp_out, float* entropy_out, float* lse_out, int64_t* stats, int16_t* ids, float* l) {
+    const EnvList e = env_list(offsets, cap, b);
+    float lp = 0.f, h = 0.f, lse = -CUDART_INF_F;
+    bool count = false;
+    if (e.n < 0) {
+        lp = h = lse = CUDART_NAN_F;
+        count = true;
+    } else if (e.n > 0) {
+        bool nan;
+        const float m = src.gather(actions, e.lo, e.n, b, ids, l, lane, nan);
+        float wz = 0.f;
+        const float S = nan ? CUDART_NAN_F : weight_pass(l, e.n, m, 1.f, lane, wz);
+        const float logS = logf(S);
+        const int want = chosen[b];
+        int c = -1;
+        for (int base = 0; base < e.n && c < 0; base += 32) {
+            const unsigned hit = __ballot_sync(kFull, base + lane < e.n && ids[base + lane] == want);
+            if (hit) c = base + __ffs(hit) - 1;
+        }
+        lse = m + logS;
+        h = logS - wz / S;
+        lp = c >= 0 ? (l[c] - m) - logS : -CUDART_INF_F;
+        count = c < 0 || S != S;                           // an id off the list, or no softmax (S = NaN): counted once
+    }
+    if (lane == 0) {
+        if (count && stats) atomicAdd((unsigned long long*)&stats[7], 1ull);
+        logp_out[b] = lp;
+        entropy_out[b] = h;
+        if (lse_out) lse_out[b] = lse;
+    }
+}
+
 template <int DT>
 __global__ void __launch_bounds__(kWarps * 32) k_policy_logprob(const int32_t* __restrict__ offsets,
                                                                 const uint64_t* __restrict__ actions, long long cap,
@@ -186,35 +242,40 @@ __global__ void __launch_bounds__(kWarps * 32) k_policy_logprob(const int32_t* _
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int b = blockIdx.x * kWarps + w;
     if (b >= B) return;
+    logprob_env(DenseLogits<DT>{logits, ld}, b, lane, offsets, actions, cap, chosen, logp_out, entropy_out, lse_out, stats,
+                sids[w], slog[w]);
+}
+
+// The gradient of env b at its legal entries, g_lp (1[id = chosen] - p) - g_ent p (log p + H), into g[0 .. n) with the
+// ids in ids[0 .. n); returns n (0 for an empty, cut or dropped list).
+template <class Src>
+DDZ_DEV int grad_env(const Src& src, int b, int lane, const int32_t* __restrict__ offsets,
+                     const uint64_t* __restrict__ actions, long long cap, const int32_t* __restrict__ chosen,
+                     const float* __restrict__ lse_in, const float* __restrict__ grad_logp,
+                     const float* __restrict__ grad_entropy, int16_t* ids, float* g) {
     const EnvList e = env_list(offsets, cap, b);
-    float lp = 0.f, h = 0.f, lse = -CUDART_INF_F;
-    bool count = false;
-    if (e.n < 0) {
-        lp = h = lse = CUDART_NAN_F;
-        count = true;
-    } else if (e.n > 0) {
+    const int n = max(e.n, 0);                             // a cut or dropped list gets a zero gradient
+    if (n > 0) {
         bool nan;
-        const float m = gather_logits<DT>(actions, e.lo, e.n, logits, (size_t)b * (size_t)ld, sids[w], slog[w], lane, nan);
-        float wz = 0.f;
-        const float S = nan ? CUDART_NAN_F : weight_pass(slog[w], e.n, m, 1.f, lane, wz);
-        const float logS = logf(S);
-        const int want = chosen[b];
-        int c = -1;
-        for (int base = 0; base < e.n && c < 0; base += 32) {
-            const unsigned hit = __ballot_sync(kFull, base + lane < e.n && sids[w][base + lane] == want);
-            if (hit) c = base + __ffs(hit) - 1;
+        src.gather(actions, e.lo, n, b, ids, g, lane, nan);
+        const float lse = lse_in[b];
+        const float glp = grad_logp ? grad_logp[b] : 0.f, gent = grad_entropy ? grad_entropy[b] : 0.f;
+        float plp = 0.f;                                   // H = -sum p log p
+        for (int i = lane; i < n; i += 32) {
+            const float lq = g[i] - lse, p = expf(lq);
+            if (p > 0.f) plp += p * lq;
         }
-        lse = m + logS;
-        h = logS - wz / S;
-        lp = c >= 0 ? (slog[w][c] - m) - logS : -CUDART_INF_F;
-        count = c < 0 || S != S;                           // an id off the list, or no softmax (S = NaN): counted once
+        const float H = -warp_sum(plp);
+        const int want = chosen[b];
+        for (int i = lane; i < n; i += 32) {
+            const float lq = g[i] - lse, p = expf(lq);
+            float v = glp * ((ids[i] == want ? 1.f : 0.f) - p);
+            if (p > 0.f) v -= gent * p * (lq + H);
+            g[i] = v;
+        }
+        __syncwarp();
     }
-    if (lane == 0) {
-        if (count && stats) atomicAdd((unsigned long long*)&stats[7], 1ull);
-        logp_out[b] = lp;
-        entropy_out[b] = h;
-        if (lse_out) lse_out[b] = lse;
-    }
+    return n;
 }
 
 // The gradient row of env b over all 13 551 ids, written once: g_lp (1[id = chosen] - p) - g_ent p (log p + H) on the
@@ -250,28 +311,8 @@ __global__ void __launch_bounds__(kWarps * 32) k_policy_logprob_backward(const i
     if (b >= B) return;
     int16_t* ids = sids[w];
     float* g = sg[w];
-    const EnvList e = env_list(offsets, cap, b);
-    const int n = max(e.n, 0);                             // a cut or dropped list gets a zero row
-    if (n > 0) {
-        bool nan;
-        gather_logits<DT>(actions, e.lo, n, logits, (size_t)b * (size_t)ld, ids, g, lane, nan);
-        const float lse = lse_in[b];
-        const float glp = grad_logp ? grad_logp[b] : 0.f, gent = grad_entropy ? grad_entropy[b] : 0.f;
-        float plp = 0.f;                                   // H = -sum p log p
-        for (int i = lane; i < n; i += 32) {
-            const float lq = g[i] - lse, p = expf(lq);
-            if (p > 0.f) plp += p * lq;
-        }
-        const float H = -warp_sum(plp);
-        const int want = chosen[b];
-        for (int i = lane; i < n; i += 32) {
-            const float lq = g[i] - lse, p = expf(lq);
-            float v = glp * ((ids[i] == want ? 1.f : 0.f) - p);
-            if (p > 0.f) v -= gent * p * (lq + H);
-            g[i] = v;
-        }
-        __syncwarp();
-    }
+    const int n = grad_env(DenseLogits<DT>{logits, ld}, b, lane, offsets, actions, cap, chosen, lse_in, grad_logp,
+                           grad_entropy, ids, g);
     char* row = reinterpret_cast<char*>(grad) + (size_t)b * (size_t)grad_ld * kEsz;
     const int head = (int)(((0u - (uint32_t)reinterpret_cast<uintptr_t>(row)) & 15u) / kEsz);   // elements before a boundary
     const int nmid = (DDZ_NUM_ACTION_IDS - head) / kSpan, tail = head + kSpan * nmid;

@@ -21,7 +21,7 @@ import torch
 
 from .agent import BatchedGreedyPolicy
 from .env import VARIANT_CHANNELS, random_deals
-from .policy import _sample as policy_sample
+from .policy import HeadedPolicy, _sample as policy_sample
 from .trainer import PackedReplayBuffer, ReplayBuffer, TransitionCollector, td_step
 
 # config.py:7-14
@@ -109,8 +109,9 @@ class BatchedGame:
     or with "determinizations": 0 the full-information search.uct_search, which sees every hand.
     policy_dict (optional) seats a fixed-head policy: role -> a module (on the game's device) that maps the env's face
     [B, C, 15, 4] to logits [B, 13551] over the action ids; that role samples its move from the softmax over its legal ids
-    (policy.policy_sample) at temperature `policy_temperature` (1.0; compete plays 0, the argmax).  Learning stays with the
-    caller.  A role has a net, a search entry or a policy entry, never two.
+    (policy.policy_sample) at temperature `policy_temperature` (1.0; compete plays 0, the argmax).  A policy.HeadedPolicy
+    (trunk + LinearPolicyHead) is sampled through head.sample(env, trunk(face)), without the dense logits.  Learning stays
+    with the caller.  A role has a net, a search entry or a policy entry, never two.
     replay="packed" keeps the learning roles' transitions as packed states and moves (trainer.PackedReplayBuffer, 176 B a
     transition instead of 2 * 240 * (C + 1) + 8 B): `dqns_dict[role]` is then called with the extra keyword replay="packed".
     Set the capacity through the DQN class, e.g. functools.partial(BatchedDQN, replay_size=10_000_000)."""
@@ -246,10 +247,15 @@ class BatchedGame:
         for role, module in self.policy_dict.items():
             mine = (seat == ROLE_INDEX[role]) & live
             if bool(mine.any()):
-                with torch.no_grad():
-                    logits = module(env.face)
                 # record=False: a -1 (nothing to draw from) is counted once, as the step's illegal choice
-                k = policy_sample(env, logits, self.policy_temperature, self._search_seed, mine, record=False)[0]
+                if isinstance(module, HeadedPolicy):              # the head at the legal ids only, no dense logits
+                    with torch.no_grad():
+                        h = module.trunk(env.face)
+                    k = module.head._sample(env, h, self.policy_temperature, self._search_seed, mine, record=False)[0]
+                else:
+                    with torch.no_grad():
+                        logits = module(env.face)
+                    k = policy_sample(env, logits, self.policy_temperature, self._search_seed, mine, record=False)[0]
                 choice = torch.where(mine, k.to(torch.int64), choice)
         was_done = env.is_done.clone()
         env.step(choice.to(torch.int32))

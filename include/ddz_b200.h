@@ -44,7 +44,9 @@ extern "C" {
 
 #define DDZ_ABI_VERSION 3   /* 3: ddz_mcts_moves, ddz_playout_pruned, ddz_q_features (+ ddz_uct_search, ddz_uct_workspace_bytes,
                             * ddz_determinize, ddz_uct_pool, ddz_encode_face_gather, ddz_move_ids, ddz_moves_of_ids, ddz_legal_mask,
-                            * ddz_policy_sample, ddz_policy_logprob, ddz_policy_logprob_backward:
+                            * ddz_policy_sample, ddz_policy_logprob, ddz_policy_logprob_backward, ddz_policy_linear_logits,
+                            * ddz_policy_linear_sample, ddz_policy_linear_logprob, ddz_policy_linear_backward,
+                            * ddz_policy_linear_workspace_bytes, ddz_policy_linear_grad_weight:
                             * new entry points only, backward compatible).  2: ddz_mpipe_*, ddz_set_tile_order, ddz_prob_form; cut lists are played
                             * from their visible part */
 #define DDZ_MAX_LEGAL 512  /* upper bound of legal moves of one decision (worst known hand: 497) */
@@ -480,6 +482,69 @@ int ddz_policy_logprob(const int32_t* offsets, const uint64_t* actions_u64, int6
 int ddz_policy_logprob_backward(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* logits,
                                 int dtype, int64_t ld, const int32_t* ids, const float* lse, const float* grad_logp,
                                 const float* grad_entropy, void* grad_logits, int64_t grad_ld, int B, void* stream);
+
+/* Linear policy heads evaluated only at the legal ids: the fixed-head policies above for a last layer
+ * logit(b, id) = W[id] . h_b + bias[id], computed from the hidden vector instead of read from a [B, 13551] logits tensor.
+ *   hidden  B rows of H elements, row b at hidden + b * ld elements;
+ *   weight  [DDZ_NUM_ACTION_IDS][H], contiguous (nn.Linear's layout: row id holds the weights of action id `id`);
+ *   bias    [DDZ_NUM_ACTION_IDS], or NULL for 0;
+ *   dtype   of all three: DDZ_DTYPE_F32 or DDZ_DTYPE_BF16 (widened exactly; all arithmetic is float);
+ *   H       a positive multiple of 16 bytes' worth of elements (4 in float, 8 in bfloat16), at most 1024; ld >= H with the
+ *           same granularity; hidden and weight 16-byte aligned, bias aligned to its element.
+ * The legal logit of an entry is computed by one function, the same in every entry point, at every B and in every launch:
+ * with the whole warp on one entry, lane k sums the products of the 16-byte pieces k, k + 32, ... of W[id] and h_b (pieces
+ * in increasing order, elements in increasing order, each a float fma), the 32 lane sums are added by the xor butterfly
+ * (distances 16, 8, 4, 2, 1), and bias[id] is added last (not at all when bias is NULL).  An entry that is not a move gets
+ * -inf, as in the dense gather.  Lists, capacity, env_mask, finished envs, cut and dropped lists, stats[7], the sticky bit,
+ * temperature and the Philox key follow ddz_policy_sample / ddz_policy_logprob / ddz_policy_logprob_backward word for word;
+ * the legal logits are then reduced by the same code, so the outputs are those of the dense entry points on a row holding
+ * these logits at the legal ids, bit for bit.
+ *
+ * ddz_policy_linear_logits: out float[cap], parallel to actions_u64: the legal logit of every stored entry.  A cut or dropped
+ * list gets NaN at its stored entries and one count in stats[7] (stats may be NULL).
+ * ddz_policy_linear_sample: ddz_policy_sample with the logits of the head; (hidden .. ld) in place of (logits, dtype, ld).
+ * ddz_policy_linear_logprob: ddz_policy_logprob with the logits of the head (logp, entropy, optional lse).
+ * ddz_policy_linear_backward: the per-env part of the gradient of ddz_policy_linear_logprob's outputs, given its lse:
+ *   grad_legal float[cap] in CSR order = the values ddz_policy_logprob_backward writes at the legal ids, exactly 0 at the
+ *              stored entries of a cut or dropped list;
+ *   grad_hidden [B][ld_g] (the first H elements of a row; ld_g >= H with H's granularity, 16-byte aligned) in the dtype of the
+ *              head: sum_i grad_legal_i * W[id_i] over the env's list, each element summed in list order (float fma);
+ *              exactly 0 for an empty, cut or dropped list.
+ * ddz_policy_linear_grad_weight: the weight and bias gradients from grad_legal, without atomics:
+ *   grad_weight[id] = sum over the entries e of id of grad_legal[e] * hidden[env(e)],   grad_bias[id] = sum of grad_legal[e]
+ *   ([DDZ_NUM_ACTION_IDS][H] contiguous, 16-byte aligned, and [DDZ_NUM_ACTION_IDS] or NULL; the dtype of the head).  Every
+ *   row and bias element is written exactly once; an id with no entry gets exact zeros.  Inputs:
+ *     n           the number of entries (n <= offsets[B] and <= the capacity the lists were written with);
+ *     order       int32[n]: the entry indices 0 .. n-1 sorted by their id, stable (a list's entries keep env order within
+ *                 an id); entries that are not moves, if any, last;
+ *     id_offsets  int32[DDZ_NUM_ACTION_IDS + 1]: id_offsets[x] = the first position in order of id x, id_offsets[0] = 0;
+ *                 positions from id_offsets[DDZ_NUM_ACTION_IDS] on are ignored;
+ *     workspace   ddz_policy_linear_workspace_bytes(n, H) bytes, 16-byte aligned (nothing to initialise).
+ *   The env of an entry is found in offsets.  The sums run over `order` cut into chunks of 128 positions: within a chunk
+ *   in position order, then the chunk partials of an id in chunk order -- an order fixed by the inputs, so two calls give
+ *   the same bits, and a long segment (the pass, id 0) is spread over many warps.
+ * NULL offsets / hidden / weight / outputs (grad_bias, lse and the two upstream gradients may be NULL; out and grad_legal
+ * only with cap = 0), actions_u64 NULL with cap > 0, cap < 0 or n < 0, B <= 0, an unknown dtype, H or ld out of range or
+ * not whole 16-byte pieces, a misaligned row, a temperature that is negative, NaN or infinite, or order / id_offsets /
+ * grad_legal / workspace NULL with n > 0: DDZ_E_ARG before any CUDA call. */
+int ddz_policy_linear_logits(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* hidden,
+                             const void* weight, const void* bias, int dtype, int H, int64_t ld, float* out, int64_t* stats,
+                             int B, void* stream);
+int ddz_policy_linear_sample(void* state, const int32_t* offsets, const uint64_t* actions_u64, int64_t cap,
+                             const void* hidden, const void* weight, const void* bias, int dtype, int H, int64_t ld,
+                             float temperature, uint64_t seed, uint64_t env0, uint32_t stepno, const uint8_t* env_mask,
+                             int32_t* choice, int32_t* ids, float* logp, float* entropy, int64_t* stats, int B, void* stream);
+int ddz_policy_linear_logprob(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* hidden,
+                              const void* weight, const void* bias, int dtype, int H, int64_t ld, const int32_t* ids,
+                              float* logp, float* entropy, float* lse, int64_t* stats, int B, void* stream);
+int ddz_policy_linear_backward(const int32_t* offsets, const uint64_t* actions_u64, int64_t cap, const void* hidden,
+                               const void* weight, const void* bias, int dtype, int H, int64_t ld, const int32_t* ids,
+                               const float* lse, const float* grad_logp, const float* grad_entropy, float* grad_legal,
+                               void* grad_hidden, int64_t ld_g, int B, void* stream);
+size_t ddz_policy_linear_workspace_bytes(int64_t n, int H);   /* 0 when n <= 0 or H is out of range */
+int ddz_policy_linear_grad_weight(const int32_t* offsets, int64_t n, const void* hidden, int dtype, int H, int64_t ld,
+                                  const float* grad_legal, const int32_t* order, const int32_t* id_offsets,
+                                  void* grad_weight, void* grad_bias, void* workspace, int B, void* stream);
 
 #ifdef __cplusplus
 }
